@@ -2,7 +2,7 @@
 """
 bench.py -- NUTS leapfrog-steps x chains / s, cubic-2 PolyModel surrogate, d=26 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one complete NUTS run (n_iter=1500, n_warmup=500: reference defaults, sample_trace.py:499-512)
@@ -29,6 +29,8 @@ tensor cores: batched logp + gradient (bfb_lik_dmma.cu) and a 4096-chain NUTS ru
              the reference arm (the port when baseline/_ref is missing; the line says which).
   extras (N = 1 unless noted): more_chains, team_kernel, pair_kernel, hmc_kernel, eval_kernel, pipeline_kernel, config3 (64-D cubic-3),
              fit_sweep (d = 32 cubic-2, N = 1e4 .. 1e7 rows; at N > 1 GPUs rows sharded + the NCCL all-reduce timed).
+  --dump-outputs DIR : the outputs of the last timed step as DIR/<name>.npy (see dump_outputs), to compare two builds; with
+             N > 1 GPUs only rank 0 writes, so the files cover its own chains, 1/N of the step.
 """
 import argparse
 import json
@@ -393,17 +395,42 @@ def fit_sweep(torch, dist, dev, rank, world, peak_dmma=None):
                 rows=rows)
 
 
+def dump_outputs(out_dir, d_out, total_tree_size, C, max_bytes=64 * 10**6, seed=0):
+    """Writes what the last timed step handed back: every output array of sampler_run, laid out [chain, iteration(, dim)],
+    for a seeded sample of whole chains (all 4096 chains are 1.8 GB; the sample fits max_bytes), plus its total_tree_size.
+    Integer statistics are stored as float64 (exact).  The inputs and the chain sample depend only on the arguments, so two
+    builds run with the same arguments can be compared file by file.  Called on rank 0 only: with several GPUs the files
+    cover rank 0's C chains (and their total_tree_size), not the other ranks' share of the step."""
+    import torch
+    bytes_per_chain = 8 * N_ITER * (N_DIM + len(d_out) - 1)         # float64 samples + one float64 per statistic
+    n_keep = min(C, (max_bytes - 4096) // bytes_per_chain)           # 4096: the .npy headers
+    chains = np.sort(np.random.default_rng(seed).choice(C, size=n_keep, replace=False))
+    idx = torch.from_numpy(chains).to(d_out['samples'].device)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in d_out.items():
+        a = v.view(C, N_ITER, N_DIM) if k == 'samples' else v.view(C, N_ITER)
+        np.save(os.path.join(out_dir, k + '.npy'), a.index_select(0, idx).to(torch.float64).cpu().numpy())
+    np.save(os.path.join(out_dir, 'total_tree_size.npy'), np.array(float(total_tree_size)))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=5)
+    ap.add_argument('--steps', type=int, default=5, help='timed steps (at least 1)')
     ap.add_argument('--warmup', type=int, default=3)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy; with several GPUs only rank 0 '
+                         'writes, covering its own chains (see dump_outputs)')
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--chains-per-gpu', type=int, default=CHAINS_PER_GPU)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--cpu-budget', type=float, default=15.)
     ap.add_argument('--no-extras', action='store_true', help='skip the more_chains / eval_kernel supplementary measurements')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 implementation')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local = int(os.environ.get('LOCAL_RANK', 0))
@@ -517,6 +544,8 @@ def main():
         kern_ms.append(kms)
     launches = h.launch_count() - l0
     kernel_family = h.sampler_last_path()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out, lv, C)
     # device time of the timed steps: CUDA events around the kernel on the launching stream (+ the reset copies,
     # which the wall clock above includes); report the event time, max over ranks
     dev_ms = float(sum(kern_ms))

@@ -1,4 +1,5 @@
 """Nested dict <-> flat .npz helpers shared by tests/ and tests/golden/make_golden.py."""
+import hashlib
 import os
 import numpy as np
 
@@ -45,6 +46,14 @@ def unflatten(flat):
         return {k: fix(v) for k, v in node.items()}
 
     return fix(root)
+
+
+def draws_digest(u, z):
+    """sha256 of a run's uniform and normal draws (float64, little-endian): pins draws a golden file regenerates instead of
+    storing them"""
+    h = hashlib.sha256(np.ascontiguousarray(u, '<f8').tobytes())
+    h.update(np.ascontiguousarray(z, '<f8').tobytes())
+    return h.hexdigest()
 
 
 def save(name, d):

@@ -624,6 +624,9 @@ def make_pipeline():
     Xt = np.array([den.from_original(x) for x in Xo])
     x0 = np.array([den.from_original(x) for x in xf[30:33] * 0.5])
     finish('multi_output_bound_transform_decay', den, dict(d=d, cinv=cinv, c0=0.3), Xt, x0, 2303, n_iter=40, n_warmup=20)
+    for c in cases:          # trees 8 doublings deep use 1.5 MB of draws: kept as a digest, the test regenerates them
+        r = c['result']
+        r['draws_sha256'] = gio.draws_digest(r.pop('draws_u'), r.pop('draws_z'))
     gio.save('pipeline_ext.npz', dict(cases=cases))
 
 

@@ -202,8 +202,12 @@ def test_pipeline_extended_case(oracle):
         assert _close(lp, c['logp'], 1e-11), c['name']
         assert _close(gr, c['grad'], 1e-11), c['name']
         r = c['result']
+        # the reference ran on the oracle's Philox streams of (seed, chain): regenerated here, pinned by their digest
+        nmax = int(np.max(r['n_draws'])) + 4
+        U, Z = map(np.array, zip(*[oracle.rng_fill(c['seed'], i, 0, nmax) for i in range(len(r['n_draws']))]))
+        assert gio.draws_digest(U, Z) == r['draws_sha256'], c['name']
         out = od.run('NUTS', {k: int(v) for k, v in c['trace_kw'].items()}, c['x0'], float(r['step0']), r['var0'],
-                     draws_u=r['draws_u'], draws_z=r['draws_z'])
+                     draws_u=U, draws_z=Z)
         assert np.all(out['status'] == 0) and np.array_equal(out['n_draws'], r['n_draws'])
         for k in INT_STATS:
             assert np.array_equal(out[k], r[k].astype(np.int32)), (c['name'], k)
