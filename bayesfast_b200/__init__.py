@@ -10,8 +10,9 @@ from .poly import PolyConfig, PolyModel
 from .density import Density, GaussianLikelihood, GaussianPrior
 from .sample_trace import NTrace, HTrace, TNTrace, THTrace, TraceTuple, SampleTrace
 from .sample import sample
+from .diag import diagnostics
 from . import random
 
 __all__ = ['PolyConfig', 'PolyModel', 'Density', 'GaussianLikelihood', 'GaussianPrior', 'NTrace', 'HTrace', 'TNTrace', 'THTrace', 'TraceTuple', 'SampleTrace', 'sample',
-           'random']
+           'diagnostics', 'random']
 __version__ = '0.1.0'

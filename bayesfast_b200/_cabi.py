@@ -48,7 +48,8 @@ class RunOut(C.Structure):
 
 
 class RunOpts(C.Structure):
-    _fields_ = [('skip', C.c_int32), ('thin', C.c_int32), ('mean', C.c_void_p), ('cov', C.c_void_p)]
+    _fields_ = [('skip', C.c_int32), ('thin', C.c_int32), ('mean', C.c_void_p), ('cov', C.c_void_p),
+                ('diag_from', C.c_int32), ('diag', C.c_void_p)]
 
 
 FLOAT_STATS = ('logp', 'energy', 'mean_tree_accept', 'step_size', 'step_size_bar', 'energy_change',
@@ -110,6 +111,8 @@ def lib():
                     ('bfb_fit_solve', [C.c_void_p, _dp, _dp], C.c_int),
                     ('bfb_fit_moments', [C.c_void_p, _dp, _dp], C.c_int),
                     ('bfb_fit_max_beta', [C.c_void_p, C.c_void_p, C.c_int64, _dp, _dp, C.POINTER(C.c_double), C.c_void_p, C.c_int], C.c_int),
+                    ('bfb_chain_diagnostics', [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int,
+                                               C.c_void_p], C.c_int),
                     ):
                 if hasattr(L, name):
                     f = getattr(L, name)
@@ -280,11 +283,12 @@ class Handle:
             check(self._L.bfb_sampler_init(self._h, C.byref(c), nc, _d(x0), _d(step0), _d(var0), _d(mean0)))
         self.n_chain = nc
 
-    def sampler_run(self, sampler, n_iter, out_ptrs=None, fields=None, skip=0, thin=1, summaries=False):
+    def sampler_run(self, sampler, n_iter, out_ptrs=None, fields=None, skip=0, thin=1, summaries=False, diag_from=None):
         """Host outputs (default): returns dict of numpy arrays [C, n_keep(, n)], n_keep = ceil((n_iter - skip) / thin):
         the records of the first `skip` iterations are not produced, of the rest every thin-th is kept ('iters': their
         iteration index within this call).  summaries: 'mean' [n] and 'cov' [n, n] of the samples of all iterations after
-        `skip` over all chains, accumulated on the device (bfb_sampler_run_ex).
+        `skip` over all chains, accumulated on the device (bfb_sampler_run_ex).  diag_from: 'diag_partials' [n, L + 3] of the
+        split-R-hat / ESS diagnostics over iterations diag_from .. n_iter - 1, L = (n_iter - diag_from) // 2 (bfb_chain_diagnostics).
         out_ptrs: dict name -> device pointer (int) for device-resident outputs, laid out [C, n_iter - skip(, n)]."""
         ro = RunOut()
         res = {}
@@ -312,6 +316,9 @@ class Handle:
         if summaries:
             res['mean'], res['cov'] = np.empty(n), np.empty((n, n))
             op.mean, op.cov = res['mean'].ctypes.data, res['cov'].ctypes.data
+        if diag_from is not None:
+            res['diag_partials'] = np.empty((n, (int(n_iter) - int(diag_from)) // 2 + 3))
+            op.diag_from, op.diag = int(diag_from), res['diag_partials'].ctypes.data
         tot = C.c_int64(0)
         check(self._L.bfb_sampler_run_ex(self._h, SAMPLER_CODE[sampler.upper()], int(n_iter), C.byref(ro), loc,
                                          C.byref(op), C.byref(tot)))
@@ -380,6 +387,13 @@ class Handle:
             res['final_var'] = cov
             res['chol_error'] = ce
         return res
+
+    def chain_diagnostics(self, x, C_, T, t0, N, n, loc):
+        """partials [n, N // 2 + 3] of bfb_chain_diagnostics; x: host array (loc BFB_HOST) or device pointer (BFB_DEVICE)"""
+        P = np.empty((int(n), int(N) // 2 + 3))
+        ptr = x.ctypes.data if loc == BFB_HOST else int(x)
+        check(self._L.bfb_chain_diagnostics(self._h, ptr, int(C_), int(T), int(t0), int(N), int(n), loc, P.ctypes.data))
+        return P
 
     def last_kernel_ms(self):
         ms = C.c_float(0)

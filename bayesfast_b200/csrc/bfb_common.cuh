@@ -182,10 +182,15 @@ struct bfb_context {
     double *t_u;
     // fit
     FitState *fit;
+    // chain diagnostics (bfb_diag.cu): device workspace, grown on demand
+    double *diag_ws;
+    size_t diag_ws_len;
 };
 
 int bfb_upload_model(bfb_context *h);          // (re)build the device tables from configs/packed
 void bfb_free_list(std::vector<void *> &v);
+// queue the split-R-hat / ESS partials of device draws x [C, T, n], kept range t0 .. t0 + N, on h->stream (bfb_diag.cu)
+int bfb_diag_enqueue(bfb_context *h, const double *x, int64_t C, int64_t T, int64_t t0, int64_t N, int n, const double **dev_partials);
 
 // ----------------------------------------------------------------------------------------------
 // warp helpers

@@ -11,14 +11,11 @@
 //
 // Outputs that are served by the same set of configs (same recipe row, poly.py:298-337) share one Gram.
 #include "bfb_common.cuh"
+#include "bfb_gram.cuh"
 #include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <map>
-
-#define TS 64          // Gram tile (features) per CTA
-#define KC 32          // rows per pipeline stage
-#define LDP (TS + 4)   // padded leading dimension: conflict-free DMMA fragment loads (LDP % 16 == 4)
 
 // temporary device allocations of one call: freed on every return path (the error paths used to leak them)
 struct TmpList : std::vector<void *> {
@@ -57,12 +54,6 @@ void bfb_fit_free(bfb_context *h)
 // ----------------------------------------------------------------------------------------------
 // Gram kernel
 // ----------------------------------------------------------------------------------------------
-__device__ __forceinline__ void dmma884(double &d0, double &d1, double a, double b)
-{
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
-}
-
 // One CTA = one 64 x 64 tile (ti <= tj) of the Gram over one chunk of rows.  Per stage of KC rows:
 //   1. the x rows are staged in shared memory with a constant-1 column appended at index n, so that a monomial with
 //      fewer than three factors needs no branch (missing factors index the 1);
@@ -147,19 +138,7 @@ __global__ void __launch_bounds__(128) gram_kernel(const double *__restrict__ x,
             }
         }
         __syncthreads();
-#pragma unroll
-        for (int kk = 0; kk < KC / 4; ++kk) {
-            const int krow = kk * 4 + (lane & 3);
-            double af[4], bf[4];
-#pragma unroll
-            for (int a = 0; a < 4; ++a) af[a] = phiI[krow * LDP + 32 * wm + 8 * a + (lane >> 2)];
-#pragma unroll
-            for (int b = 0; b < 4; ++b) bf[b] = phiJ[krow * LDP + 32 * wn + 8 * b + (lane >> 2)];
-#pragma unroll
-            for (int a = 0; a < 4; ++a)
-#pragma unroll
-                for (int b = 0; b < 4; ++b) dmma884(acc[a][b][0], acc[a][b][1], af[a], bf[b]);
-        }
+        gram_tile_mma(phiI, phiJ, lane, wm, wn, acc);
     }
     double *out = ws + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * (TS * TS);
 #pragma unroll

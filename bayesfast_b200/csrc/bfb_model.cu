@@ -64,6 +64,7 @@ extern "C" int bfb_create(int device, bfb_handle *out)
     h->dense_metric = false;
     h->lik_tab = nullptr; h->lik_nr = 0; h->last_eval_path = -1;
     h->fit = nullptr;
+    h->diag_ws = nullptr; h->diag_ws_len = 0;
     h->t_base = nullptr; h->t_logxi = 0.; h->t_u = nullptr;
     h->gstack = nullptr;
     h->gstack_len = 0;
@@ -98,6 +99,7 @@ extern "C" int bfb_destroy(bfb_handle h)
     bfb_free_list(h->dense_allocs);
     bfb_fit_free(h);
     if (h->gstack) cudaFree(h->gstack);
+    if (h->diag_ws) cudaFree(h->diag_ws);
     if (h->t_u) cudaFree(h->t_u);
     if (h->queue) cudaFree(h->queue);
     if (h->progress_host) cudaFreeHost(h->progress_host);

@@ -13,6 +13,7 @@
 // hmc_utils/step_size.py:10-51.  Draw order: SURVEY.md 8(a) row N-RNG; stream: include/bfb_rng.h.
 #include "bfb_common.cuh"
 #include "bfb_eval.cuh"
+#include <algorithm>
 #include <cstring>
 #include <cstdio>
 #include <cstdlib>
@@ -880,8 +881,11 @@ static int launch_run(bfb_context *h, int sampler, int n_iter, const bfb_run_out
 // Host outputs from ONE launch (the tensor-core NUTS kernel reports progress; anything else returns 1 before launching and the
 // caller falls back to the chunked launches): device buffer [C, R(, n)] per field, the host thread polls the progress word the
 // kernel writes into mapped pinned memory and queues the strided copy of every finished chunk on the copy stream.
+// diag_t0 >= 0: the diagnostics of iterations diag_t0 .. R - 1 are queued behind the kernel (they overlap the last copies), *diag_P
+// receives their device partials.
 // Returns BFB_OK when the run was done (ev1 recorded, copies complete), 1 when this path does not apply, < 0 on error.
-static int single_launch_host_outputs(bfb_context *h, int sampler, int R, void *const user[11], int n_keep)
+static int single_launch_host_outputs(bfb_context *h, int sampler, int R, void *const user[11], int n_keep, int diag_t0,
+                                      const double **diag_P)
 {
     const DevModel &M = h->dm;
     // only nuts_dmma_kernel reports progress: the same conditions as bfb_launch_nuts_dmma, default kernel selection
@@ -935,6 +939,7 @@ static int single_launch_host_outputs(bfb_context *h, int sampler, int R, void *
     if (rc) return rc;
     h->iters_done += R;
     BFB_CUDA(cudaEventRecord(h->ev1, h->stream));
+    if (diag_t0 >= 0 && (rc = bfb_diag_enqueue(h, (const double *)dptr[0], C, R, diag_t0, R - diag_t0, n, diag_P))) return rc;
     const bool rep[2] = {const_steps && user[4] != nullptr, const_steps && user[5] != nullptr};
     double *col = nullptr;                          // pinned [2][C]: the first record of the two fields
     struct ColGuard { double *&p; ~ColGuard() { if (p) cudaFreeHost(p); } } col_guard{col};
@@ -1079,7 +1084,11 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
     BFB_REQUIRE(sampler != BFB_HMC || h->scfg.n_int_step > 0, BFB_ERR_ARG, "n_int_step must be positive");
     const int skip = opts ? opts->skip : 0, thin = opts ? opts->thin : 1;
     const bool want_mom = opts && (opts->mean || opts->cov);
+    const bool want_diag = opts && opts->diag;
+    const int dfrom = want_diag ? opts->diag_from : 0;
     BFB_REQUIRE(skip >= 0 && skip <= n_iter && thin >= 1, BFB_ERR_ARG, "bfb_sampler_run_ex: need 0 <= skip <= n_iter and thin >= 1");
+    BFB_REQUIRE(!want_diag || (dfrom >= skip && n_iter - dfrom >= 4), BFB_ERR_ARG,
+                "bfb_sampler_run_ex: the diagnostics need skip <= diag_from <= n_iter - 4 (skip %d, diag_from %d, n_iter %d)", skip, dfrom, n_iter);
     BFB_REQUIRE(loc == BFB_HOST || (thin == 1 && !want_mom), BFB_ERR_ARG, "bfb_sampler_run_ex: thinning and summaries need host outputs");
     BFB_CUDA(cudaSetDevice(h->device));
     const int64_t C = h->cs.C;
@@ -1097,16 +1106,43 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
     }
     const int R = n_iter - skip;            // iterations with records
     const int n_keep = (R + thin - 1) / thin;
+    // diagnostics: iterations dfrom .. n_iter - 1 are draws diag_t0 .. of diag_src [C, diag_T, n]; diag_buf holds them when no
+    // buffer of the run does
+    const int Rd = n_iter - dfrom;
+    const double *diag_P = nullptr, *diag_src = nullptr;
+    int64_t diag_T = 0, diag_t0 = 0;
+    double *diag_buf = nullptr;
+    struct DiagGuard { double *&p; ~DiagGuard() { if (p) cudaFree(p); } } diag_guard{diag_buf};
+    auto alloc_diag_buf = [&](int iters) -> int {
+        const size_t bytes = sizeof(double) * (size_t)C * (size_t)iters * (size_t)n;
+        const cudaError_t e = cudaMalloc((void **)&diag_buf, bytes);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            diag_buf = nullptr;
+            bfb_set_error("bfb_sampler_run_ex: the diagnostics need the samples of %d iterations x %lld chains resident on the device, "
+                          "a %.2f GB buffer that cannot be allocated (%s)", iters, (long long)C, 1e-9 * (double)bytes, cudaGetErrorString(e));
+            return BFB_ERR_CUDA;
+        }
+        return BFB_OK;
+    };
     int single_rc = 1;
-    if (R >= 64 && loc == BFB_HOST && sampler == BFB_NUTS && !h->dense_metric && thin == 1 && !want_mom && !getenv("BFB200_E2E_MULTI_LAUNCH")) {
-        single_rc = single_launch_host_outputs(h, sampler, R, user, n_keep);
+    if (R >= 64 && loc == BFB_HOST && sampler == BFB_NUTS && !h->dense_metric && thin == 1 && !want_mom && (!want_diag || user[0]) &&
+        !getenv("BFB200_E2E_MULTI_LAUNCH")) {
+        single_rc = single_launch_host_outputs(h, sampler, R, user, n_keep, want_diag ? dfrom - skip : -1, &diag_P);
         if (single_rc < 0) return single_rc;
     }
     if (R == 0) {
     } else if (loc == BFB_DEVICE) {
-        int rc = launch_run(h, sampler, R, *out);
+        bfb_run_out dev = *out;
+        if (want_diag && !dev.samples) {
+            int rc = alloc_diag_buf(R);
+            if (rc) return rc;
+            dev.samples = diag_buf;
+        }
+        int rc = launch_run(h, sampler, R, dev);
         if (rc) return rc;
         h->iters_done += R;
+        diag_src = dev.samples; diag_T = R; diag_t0 = dfrom - skip;
     } else if (single_rc == BFB_OK) {
         // done: ONE launch for all R iterations into a device buffer laid out like the caller's arrays; the kernel reported every
         // finished chunk of iterations and the host copied it out while the kernel went on (no launch boundaries, no tails)
@@ -1122,7 +1158,7 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
         n_chunks = (R + K - 1) / K;
         size_t rec = 0;
         for (int f = 0; f < 11; ++f) if (user[f]) rec += field_bytes(f, n);
-        const bool stage_samples = want_mom && !user[0];    // the summaries need the samples even if the caller does not
+        const bool stage_samples = (want_mom || want_diag) && !user[0];    // the summaries need the samples even if the caller does not
         if (stage_samples) rec += field_bytes(0, n);
         const size_t full = rec * (size_t)C * K;
         const size_t need = full + (thin > 1 ? rec * (size_t)C * ((K + thin - 1) / thin) : 0);
@@ -1140,6 +1176,11 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
             }
         }
         const int ne = n + n * n, nb = h->sm_count * 2;
+        if (want_diag) {
+            int rc = alloc_diag_buf(Rd);
+            if (rc) return rc;
+            diag_src = diag_buf; diag_T = Rd; diag_t0 = 0;
+        }
         double *mom = nullptr;              // [n] shift | [ne] accumulators | [nb][ne] partials
         if (want_mom) {
             BFB_CUDA(cudaMalloc((void **)&mom, sizeof(double) * ((size_t)n + ne + (size_t)nb * ne)));
@@ -1170,6 +1211,13 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
                 trace_moments_partial_kernel<<<nb, 256, sizeof(double) * 32 * n, h->stream>>>((const double *)dptr[0], C * (int64_t)Kk, n, mom, mom + n + ne);
                 trace_moments_reduce_kernel<<<(ne + 127) / 128, 128, 0, h->stream>>>(mom + n + ne, nb, ne, mom + n);
                 h->launches += 2;
+            }
+            if (want_diag) {                // this chunk's iterations from dfrom on, into the resident buffer
+                const int lo = std::max(it_begin, dfrom - skip), hi = it_begin + Kk;
+                if (hi > lo)
+                    BFB_CUDA(cudaMemcpy2DAsync(diag_buf + (size_t)(lo - (dfrom - skip)) * n, sizeof(double) * n * (size_t)Rd,
+                                               (const double *)dptr[0] + (size_t)(lo - it_begin) * n, sizeof(double) * n * (size_t)Kk,
+                                               sizeof(double) * n * (size_t)(hi - lo), (size_t)C, cudaMemcpyDeviceToDevice, h->stream));
             }
             if (thin > 1) {
                 for (int f = 0; f < 11; ++f) {
@@ -1209,6 +1257,11 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
         BFB_CUDA(cudaStreamSynchronize(h->copy_stream));
     }
     if (R == 0 || loc == BFB_DEVICE) BFB_CUDA(cudaEventRecord(h->ev1, h->stream));
+    if (diag_src) {
+        int rc = bfb_diag_enqueue(h, diag_src, C, diag_T, diag_t0, Rd, n, &diag_P);
+        if (rc) return rc;
+    }
+    if (want_diag) BFB_CUDA(cudaMemcpyAsync(opts->diag, diag_P, sizeof(double) * (size_t)n * (size_t)(Rd / 2 + 3), cudaMemcpyDeviceToHost, h->stream));
     BFB_CUDA(cudaMemcpyAsync(&tt, h->cs.tree_total, sizeof(tt), cudaMemcpyDeviceToHost, h->stream));
     BFB_CUDA(cudaStreamSynchronize(h->stream));
     BFB_CUDA(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));

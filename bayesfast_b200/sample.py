@@ -8,7 +8,7 @@ import time
 
 import numpy as np
 
-from . import _cabi
+from . import _cabi, diag
 from .density import Density
 from .random import get_generator, new_seed
 from .runtime import dist_info, shard_bounds
@@ -42,6 +42,24 @@ def _out_plan(trace, i_iter, n_run, keep, thin):
 
 
 
+def _diag_from(trace, i_iter, n_run, diagnostics):
+    """first iteration of this call after the warm-up, where the diagnostics start (None: no diagnostics)"""
+    if not diagnostics:
+        return None
+    d = min(max(trace.n_warmup - i_iter, 0), n_run)
+    if n_run - d < 4:
+        raise ValueError('diagnostics=True needs at least 4 post-warm-up iterations in this call, there are {}.'.format(n_run - d))
+    return d
+
+
+def _diagnostics(res, comm, device):
+    """this call's diagnostics over all ranks' chains from the partials bfb_sampler_run_ex left in res"""
+    P = res.pop('diag_partials', None)
+    if P is None:
+        return None
+    return diag.finish(diag.combine(P, comm, device))
+
+
 def sobol_multivariate_normal(dim, size, skip=1):
     """bayesfast.utils.sobol.multivariate_normal(zeros(dim), eye(dim), size) (utils/sobol.py:48-60, utils/_sobol.pyx): the first
     `size` points after `skip` of the Joe-Kuo Sobol sequence (Gray-code order, direction numbers new-joe-kuo-6.21201), mapped through
@@ -57,7 +75,7 @@ def sobol_multivariate_normal(dim, size, skip=1):
 
 
 def sample(density, sample_trace=None, sampler='NUTS', n_run=None, parallel_backend='b200', verbose=True,
-           comm=None, fields=None, keep='all', thin=1, summaries=False):
+           comm=None, fields=None, keep='all', thin=1, summaries=False, diagnostics=False):
     """
     Sampling a surrogate density with lock-step NUTS / HMC on the GPU.
 
@@ -68,7 +86,9 @@ def sample(density, sample_trace=None, sampler='NUTS', n_run=None, parallel_back
     `keep='post_warmup'`: the records of the warm-up iterations are never written or copied (SampleTrace.get drops them
     anyway, sample_trace.py:762-787); `thin=k`: of the iterations kept only every k-th record comes back; `summaries=True`:
     mean and covariance (np.cov) of ALL samples after the dropped iterations, over this rank's chains, accumulated on the
-    device (tt.summaries).  A 4096-chain, 1500-iteration run at n = 26 brings back 1.7 GB per GPU with the defaults,
+    device (tt.summaries).  `diagnostics=True`: split-R-hat and effective sample size (bayesfast_b200.diagnostics) of the samples of
+    this call's post-warm-up iterations over all ranks' chains, whatever `fields`, `keep` and `thin` bring back, computed on the
+    device (tt.diagnostics = dict(rhat, ess)).  A 4096-chain, 1500-iteration run at n = 26 brings back 1.7 GB per GPU with the defaults,
     1.1 GB with keep='post_warmup', 0.11 GB with thin=10 on top.
 
     Returns
@@ -111,7 +131,7 @@ def sample(density, sample_trace=None, sampler='NUTS', n_run=None, parallel_back
     n = den.input_size
     rank, world, _ = dist_info(comm)
     if resume is not None:
-        return _continue(den, resume, n_run, verbose)
+        return _continue(den, resume, n_run, verbose, comm)
 
     if trace.random_generator is None:
         trace.random_generator = new_seed()
@@ -157,6 +177,8 @@ def sample(density, sample_trace=None, sampler='NUTS', n_run=None, parallel_back
     mean0 = x0 if trace._initial_mean is None else np.broadcast_to(trace._initial_mean, (Cl, n))
 
     if sampler in ('TNUTS', 'THMC'):
+        if diagnostics:
+            raise NotImplementedError('diagnostics are not available for the tempered samplers.')
         return _sample_tempered(den, trace, sampler, n_run, verbose, fields, keep, thin, summaries, seed, lo, x0, step0,
                                 dense, var0, mean0)
     h = den._sync(False)
@@ -170,14 +192,18 @@ def sample(density, sample_trace=None, sampler='NUTS', n_run=None, parallel_back
         trace._n_iter = n_run
     t0 = time.time()
     skip, thin = _out_plan(trace, 0, n_run, keep, thin)
-    res = h.sampler_run(sampler, n_run, fields=fields, skip=skip, thin=thin, summaries=summaries)
+    dfrom = _diag_from(trace, 0, n_run, diagnostics)
+    res = h.sampler_run(sampler, n_run, fields=fields, skip=skip, thin=thin, summaries=summaries, diag_from=dfrom)
     final = h.sampler_state()
     _raise_status(final['status'], lo)
+    dg = _diagnostics(res, comm, h.device)
     final['step0'], final['x_0'] = step0, x0
     arrays = _finish_arrays(den, res)
     tt = TraceTuple(trace, arrays, final, chain0=lo, device_state=h, iters=res['iters'], i_iter=n_run,
-                    out_opts=dict(fields=fields, keep=keep, thin=thin, summaries=summaries), generation=h.generation)
+                    out_opts=dict(fields=fields, keep=keep, thin=thin, summaries=summaries, diagnostics=bool(diagnostics)),
+                    generation=h.generation)
     tt.summaries = {k: res[k] for k in ('mean', 'cov') if k in res}
+    tt.diagnostics = dg
     tt.total_tree_size = res['total_tree_size']
     tt.kernel_ms = h.last_kernel_ms()
     if verbose:
@@ -249,7 +275,7 @@ def _finish_arrays(den, res):
     return arrays
 
 
-def _continue(den, tt, n_run, verbose):
+def _continue(den, tt, n_run, verbose, comm=None):
     """in-memory resume (sample.py:91-98, base_hmc.py:101-111): the chains are still resident on the device"""
     h = tt._device_state
     if h is None or h is not den._sync(False) or getattr(h, 'generation', None) != tt._generation:
@@ -264,9 +290,11 @@ def _continue(den, tt, n_run, verbose):
         trace._n_iter = tt.i_iter + n_run
     oo = tt._out_opts
     skip, thin = _out_plan(trace, tt.i_iter, n_run, oo['keep'], oo['thin'])
-    res = h.sampler_run(tt.sampler, n_run, fields=oo['fields'], skip=skip, thin=thin, summaries=oo['summaries'])
+    dfrom = _diag_from(trace, tt.i_iter, n_run, oo.get('diagnostics', False))
+    res = h.sampler_run(tt.sampler, n_run, fields=oo['fields'], skip=skip, thin=thin, summaries=oo['summaries'], diag_from=dfrom)
     final = h.sampler_state()
     _raise_status(final['status'], tt._chain0)
+    dg = _diagnostics(res, comm, h.device)
     final['step0'], final['x_0'] = tt._final['step0'], tt._final['x_0']
     new = _finish_arrays(den, res)
     arrays = {k: np.concatenate((tt._arrays[k], new[k]), axis=1) for k in new if k in tt._arrays}
@@ -274,6 +302,7 @@ def _continue(den, tt, n_run, verbose):
                      iters=np.concatenate((tt._iters, tt.i_iter + res['iters'])), i_iter=tt.i_iter + n_run, out_opts=oo,
                      generation=tt._generation)
     out.summaries = {k: res[k] for k in ('mean', 'cov') if k in res}       # of this call's iterations
+    out.diagnostics = dg                                                      # of this call's post-warm-up iterations
     out.total_tree_size = tt.total_tree_size + res['total_tree_size']
     out.kernel_ms = h.last_kernel_ms()
     if verbose:

@@ -476,6 +476,7 @@ class TraceTuple:
         self._i_iter = n_rec if i_iter is None else int(i_iter)
         self.total_tree_size = 0
         self.summaries = {}
+        self.diagnostics = None                 # sample(diagnostics=True): dict(rhat, ess) of the call's post-warm-up iterations
         self._cache = {}
 
     def _arr(self, name):

@@ -184,10 +184,16 @@ int bfb_sampler_run(bfb_handle h, int sampler, int32_t n_iter, const bfb_run_out
  * skip: the records of the first `skip` iterations of this call are not written at all; thin >= 1: of the following
  * iterations every thin-th is kept, the out arrays are then [C, n_keep(, n)] with n_keep = ceil((n_iter - skip) / thin)
  * (host outputs only for thin > 1); mean [n] / cov [n,n] (host, may be NULL): mean and unbiased covariance (np.cov) of the
- * samples of ALL iterations after `skip` over all chains, accumulated on the device.  opts == NULL: bfb_sampler_run. */
+ * samples of ALL iterations after `skip` over all chains, accumulated on the device.  opts == NULL: bfb_sampler_run.
+ * diag [n, (n_iter - diag_from) / 2 + 3] (host, may be NULL): the partials of bfb_chain_diagnostics over the samples of iterations
+ * diag_from .. n_iter - 1 of this call, whatever skip, thin and out ask for; skip <= diag_from <= n_iter - 4.  They are computed on
+ * the device from the buffer the samples are staged in, or from one [C, n_iter - diag_from, n] buffer that holds them otherwise
+ * (BFB_ERR_CUDA naming the size when it cannot be allocated). */
 typedef struct {
     int32_t skip, thin;
     double *mean, *cov;
+    int32_t diag_from;
+    double *diag;
 } bfb_run_opts;
 int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, const bfb_run_out *out, int loc,
                        const bfb_run_opts *opts, int64_t *total_tree_size);
@@ -229,7 +235,16 @@ int bfb_sampler_get_state(bfb_handle h, double *final_step, double *final_var, i
 int bfb_importance_weights(bfb_handle h, const double *logp, const double *logq, int64_t N, double k_trunc,
                            double *weights, double *weights_trunc, double *stats, int loc);
 int bfb_argsort_gather(bfb_handle h, const double *a, int64_t N, const int64_t *pos, int64_t n, int64_t *out, int loc);
-/* device time of the last bfb_sampler_run / bfb_fit_accumulate / bfb_poly_eval_batch kernel(s), CUDA events
+/* Convergence diagnostics of sampled chains (replaces nothing in the reference, which leaves them to the caller; the definitions are
+ * those of Stan's and ArviZ's non-rank-normalised split-R-hat and ESS, bayesfast_b200/diag.py): x [C, T_total, n] in `loc`, draws
+ * t0 .. t0 + N - 1 of every chain (N >= 4), split into M' = 2 C half-chains of L = N / 2 draws.  partials [n, L + 3] (host) per
+ * coordinate: M' | mean of the half-chain means | sum of their squared deviations from it | the lag sums S(k) = sum over half-chains
+ * of sum_t y[t] y[t + k], k = 0 .. L - 1, of the centred half-chains y.  All are sums over chains: shards of chains combine with a
+ * pairwise (Chan) update of the first three and a sum of the rest.  The lag sums run on the FP64 tensor cores; repeated calls are
+ * bit-identical. */
+int bfb_chain_diagnostics(bfb_handle h, const double *x, int64_t C, int64_t T_total, int64_t t0, int64_t N, int n, int loc,
+                          double *partials);
+/* device time of the last bfb_sampler_run / bfb_fit_accumulate / bfb_poly_eval_batch / bfb_chain_diagnostics kernel(s), CUDA events
  * on the handle's stream, milliseconds */
 int bfb_last_kernel_ms(bfb_handle h, float *ms);
 /* number of kernels launched by this handle since creation */
