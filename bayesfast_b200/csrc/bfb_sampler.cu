@@ -1269,7 +1269,7 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
     if (getenv("BFB200_DEBUG")) {
         unsigned long long dbg[16];
         BFB_CUDA(cudaMemcpy(dbg, h->cs.tree_total, sizeof(dbg), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "[bfb200] leaves %llu warp-rounds %llu merge-sections %llu iter-end-sections %llu  ms %.3f\n", dbg[0], dbg[1], dbg[2], dbg[3], h->last_ms);
+        fprintf(stderr, "[bfb200] leaves %llu warp-rounds %llu merge-passes %llu iter-end-sections %llu  ms %.3f\n", dbg[0], dbg[1], dbg[2], dbg[3], h->last_ms);
         if (dbg[1] && h->last_path == 3)
             fprintf(stderr, "[bfb200] team kernel, leader-warp cycles per round: apply %.0f boundary %.0f leapfrog+eval %.0f owners %.0f tasks+leaf %.0f decisions %.0f command-barrier %.0f\n",
                     (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
@@ -1279,7 +1279,7 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
                     (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
                     (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1], dbg[12],
                     (double)dbg[13] / (dbg[12] ? dbg[12] : 1), (double)dbg[14] / (dbg[12] ? dbg[12] : 1), (double)dbg[15] / (dbg[12] ? dbg[12] : 1));
-        else if (dbg[1]) fprintf(stderr, "[bfb200] cycles per warp-round: boundary %.0f rng+dbl %.0f (unused) %.0f leaf-pair %.0f merges %.0f push %.0f extend %.0f | unit setup+teardown per round %.0f\n",
+        else if (dbg[1]) fprintf(stderr, "[bfb200] cycles per warp-round: boundary %.0f rng+dbl %.0f (unused) %.0f leaves %.0f merge-loop %.0f push %.0f extend %.0f | unit setup+teardown per round %.0f\n",
                             (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
                             (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1]);
     }

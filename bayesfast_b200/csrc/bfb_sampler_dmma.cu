@@ -40,10 +40,11 @@ void *bfb_pad_kernel_ref() { return (void *)bfb_pad_kernel<BFB_CODE_PAD>; }
 #endif
 
 
-// shared memory per warp, in doubles: TL q,p,g | TR q,p,g | PS | PB | stack levels (pl, pr, psum) | per-level scalars
-// [5][10][8 chains]: weight mantissa, weight exponent, proposal energy, proposal logp, proposal slot.
+// shared memory per warp, in doubles: TL q,p,g | TR q,p,g | PS | PB | stack levels 0..LS (pl, pr, psum) | per-level
+// scalars [5][10][8 chains]: weight mantissa, weight exponent, proposal energy, proposal logp, proposal slot.  Level 0 holds
+// the current subtree R; its scalars live in registers, and scalar level 0 holds the first leaf of a pair until it is merged.
 // A vector slot holds element (r, lane) at r * 32 + lane: every access is one conflict-free 256-byte row.
-__host__ __device__ inline int warp_smem_doubles(int NR, int LS) { return (8 + 3 * LS) * NR * 32 + 400; }
+__host__ __device__ inline int warp_smem_doubles(int NR, int LS) { return (11 + 3 * LS) * NR * 32 + 400; }
 
 template <int NR, int MV, int W>
 __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sampler_cfg cfg, ChainState st, RunOutDevF out,
@@ -51,6 +52,7 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
                                                               double *__restrict__ gprop, int base_iter, int chunk_iters,
                                                               int n_groups, int n_units, int *__restrict__ queue, int cpg)
 {
+    // section: setup
     using SH = DmmaShape<NR, MV>;
     constexpr int SLOT = NR * 32;
     extern __shared__ double smem[];
@@ -63,7 +65,7 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
     const int c3x = SH::C3 ? dmma_c3_doubles(NR, M.c3_kt, W) : 0;          // cubic-3 operand table, pair table, x scratch
     double *wsm = smem + SH::frag_doubles(W) + SH::MSM_DOUBLES + c3x + (size_t)wib * warp_smem_doubles(NR, LS);
     double *sTL = wsm, *sTR = wsm + 3 * SLOT, *sPS = wsm + 6 * SLOT, *sPB = wsm + 7 * SLOT, *sST = wsm + 8 * SLOT;
-    double *ssc = wsm + (8 + 3 * LS) * SLOT + gi;        // scalar (field f, level l) of this chain at ssc[(f * 10 + l) * 8]
+    double *ssc = wsm + (11 + 3 * LS) * SLOT + gi;       // scalar (field f, level l) of this chain at ssc[(f * 10 + l) * 8]
     const int n = M.n;
     const DmmaConsts K = dmma_consts(M);
 
@@ -134,24 +136,25 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
     WT Wtree; Wtree.m = 1.; Wtree.k = 0;
     int depth = 0, ileaf = 0, n_prop = 0, diverging = 0, prop_slot = 0, Rslot = 0;
     unsigned freemask = 0;
-    double Rpl[NR], Rps[NR], REp = 0., Rlpp = 0.;
+    double REp = 0., Rlpp = 0.;
     WT RW; RW.m = 0.; RW.k = 0;
-#pragma unroll
-    for (int r = 0; r < NR; ++r) Rpl[r] = Rps[r] = 0.;
     // per-chain control flags: bnd = an iteration boundary is pending (end the previous iteration unless `fresh`,
     // start the next unless done), ns_dbl = a doubling must be started
     bool bnd = !done, fresh = true, ns_dbl = false;
+    // the current subtree R (left-end p, right-end p, p_sum) is the level-0 stack entry
+    double *sR = sST;
     // scratch vectors of the boundary section alias the (then empty) level-0 stack entry
     double *sP0 = sST, *sVAR = sST + SLOT, *sQN = sST + 2 * SLOT;
 
-    // stack entry of level lvl >= 1 (level 0 lives in registers, see "two leaves per round"): the first LS in shared memory
+    // stack entry of level lvl: levels 0..LS in shared memory, deeper ones in the L2-resident buffer
     auto stack_ptr = [&](int lvl) -> double * {
-        return (lvl <= LS) ? (sST + (lvl - 1) * 3 * SLOT) : (gst + (size_t)(lvl - 1 - LS) * 3 * SLOT);
+        return (lvl <= LS) ? (sST + lvl * 3 * SLOT) : (gst + (size_t)(lvl - 1 - LS) * 3 * SLOT);
     };
 
 #pragma unroll 1
     while (__any_sync(BFB_FULL, !done)) {
         TICK(7)
+        // section: boundary
         // ================= iteration boundary: base_hmc.py:62-85, Tree.__init__ nuts.py:27-43 =================
         if (__any_sync(BFB_FULL, bnd)) {
             DBG_COUNT(dbg_iend)
@@ -302,6 +305,7 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
         const bool live = !done;
         DBG_COUNT(dbg_rounds)
         TICK(0)
+        // section: round start
         // ---- uniforms of this round: lane lg of a quad holds draws 2 (t/2 + lg) + {0, 1} of its chain ----
         const int64_t tb2 = (t >> 1) << 1;
         const double2 ub = philox_pair_ni(seed, chain_id, (uint64_t)(t >> 1) + (uint64_t)lg);
@@ -329,12 +333,12 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
             }
         }
         TICK(1)
+        // section: evaluation
         // ================= two leaves per round =================
         // A leaf with an even index is never followed by a decision (it is the left child of a level-0 merge), so a
         // round integrates a PAIR of leaves whenever the doubling has at least two: the fixed cost of a round (every
-        // section below is paid per warp, not per chain) is spread over two leapfrogs, and the level-0 merge works on
-        // registers (level 0 of the stack is never stored).  Doublings of one leaf and divergent first leaves skip the
-        // second half.
+        // section below is paid per warp, not per chain) is spread over two leapfrogs.  Doublings of one leaf and
+        // divergent first leaves skip the second half.
         const double dt = 0.5 * step;
         bool div_now = false, turn = false, did2 = false;
 #ifdef BFB_UNROLL_HALVES
@@ -372,6 +376,7 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
                     }
                 }
             }
+            // section: leaf
             const double E = 0.5 * ke2 - lp;
             // ---- leaf: Tree._single_step, nuts.py:105-132 ----
             double dE = E - E0;
@@ -385,170 +390,132 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
             }
             const WT wl = wt_from_dE(div_leaf ? 0. : dE);
             const bool okl = go && !div_leaf;
-            int nslot = 0;
             if (okl) {
                 acc_sum += wt_min1(wl);
-                nslot = __ffs(freemask) - 1;
+                const int nslot = __ffs(freemask) - 1;
                 freemask &= ~(1u << nslot);
                 double *slot = gpr + (size_t)nslot * 2 * SLOT;
                 VST(slot, q) VST(slot + SLOT, g)
+                // the leaf becomes R; the first leaf of a pair waits at scalar level 0 for the level-0 merge, and its p
+                // (left end and p_sum of R) is the left tree of that merge
+                if (half == 1) {
+                    ssc[0] = RW.m; ssc[10 * 8] = (double)RW.k; ssc[20 * 8] = REp; ssc[30 * 8] = Rlpp; ssc[40 * 8] = (double)Rslot;
+                    did2 = true;
+                } else {
+                    VST(sR, p) VST(sR + 2 * SLOT, p)
+                }
+                VST(sR + SLOT, p)
+                RW = wl; REp = E; Rlpp = lp; Rslot = nslot;
             }
             if (div_leaf) { diverging = 1; div_now = true; }
-            if (half == 0) {
-                if (okl) {
-#pragma unroll
-                    for (int r = 0; r < NR; ++r) { Rpl[r] = p[r]; Rps[r] = p[r]; }
-                    RW = wl; REp = E; Rlpp = lp; Rslot = nslot;
-                }
-            } else {
-                // ---- level-0 merge of the two leaves (nuts.py:134-178 with depth 1: only the full-span U-turn test) ----
-                double v0 = 0., v1 = 0.;
-#pragma unroll
-                for (int r = 0; r < NR; ++r) {
-                    const double ps = Rps[r] + p[r];
-                    v0 = fma(ps, var[r] * Rpl[r], v0); v1 = fma(ps, var[r] * p[r], v1);
-                }
-                double z0 = 1., z1 = 1.;
-                qsum4(v0, v1, z0, z1, lane);
-                const double um = uni(t);
-                if (okl) {
-                    t += 1;
-                    const WT tot = wt_add(RW, wl);
-                    if (!wt_select(um, tot, wl)) {               // keep the first leaf as the proposal (nuts.py:164-167)
-                        freemask |= 1u << nslot;
-                    } else {
-                        freemask |= 1u << Rslot;
-                        Rslot = nslot; REp = E; Rlpp = lp;
-                    }
-#pragma unroll
-                    for (int r = 0; r < NR; ++r) Rps[r] += p[r];
-                    RW = tot;
-                    if (v0 <= 0. || v1 <= 0.) turn = true;
-                    did2 = true;
-                }
-            }
         }
         TICK(3)
-        // ================= merges above level 0: Tree._build_subtree, nuts.py:134-178 =================
-        int lvl = 1;
-        bool need = did2 && !turn && ((ileaf >> lvl) & 1);
+        // section: merge
+        // ================= merges: Tree._build_subtree nuts.py:134-178 and Tree.extend nuts.py:45-103 =================
+        // Every live chain works through a queue, one merge per pass: the level-0 merge of a leaf pair, then the merges at
+        // levels 1, 2, ... while (ileaf >> lvl) & 1 and no U-turn, then Tree.extend if the doubling ended.  A merge combines a
+        // pending tree T with the current subtree R: T is a stack level (multinomial choice of the proposal, nuts.py:164-167)
+        // or, for the extend, the whole tree (biased progressive choice, nuts.py:81-83).  The U-turn test runs on the two
+        // trees in their order along the trajectory, X then Y, each given by the addresses of its left-end p, right-end p and
+        // p_sum; a single leaf has all three at one address.
+        int lvl = 0;
+        int mq = live ? (did2 ? 0 : 1) : 3;      // next: 0 subtree merge at lvl, 1 decide on the extend, 2 extend, 3 none
+        bool fin = false;
+        const bool right = step > 0.;
 #pragma unroll 1
-        while (__any_sync(BFB_FULL, need)) {
-            const int lv = need ? lvl : 1;
-            DBG_COUNT(dbg_merges)
-            double T1pl[NR], T1pr[NR], T1ps[NR];
-            if (__any_sync(BFB_FULL, lv > LS)) {              // a deep level somewhere in the warp: generic loads
-                const double *sp = stack_ptr(lv);
-                VLD(T1pl, sp) VLD(T1pr, sp + SLOT) VLD(T1ps, sp + 2 * SLOT)
-            } else {                                          // common case: shared-memory loads
-                const double *sp = sST + (lv - 1) * 3 * SLOT;
-                VLD(T1pl, sp) VLD(T1pr, sp + SLOT) VLD(T1ps, sp + 2 * SLOT)
+        for (;;) {
+            if (mq == 1) {
+                fin = div_now || turn || (ileaf + 1 == (1 << depth));
+                mq = (fin && !div_now && !turn) ? 2 : 3;
             }
+            const bool go = mq == 0 || mq == 2, ext = mq == 2;
+            if (!__any_sync(BFB_FULL, go)) break;
+            DBG_COUNT(dbg_merges)
+            // X, Y = stack level and R (level 0: the two leaves); extend: the whole tree and R, or R reversed and the whole tree
+            const bool leaf0 = !ext && lvl == 0, extl = ext && !right;
+            const double *tp = stack_ptr(go && !ext ? lvl : 0);
+            const double *xl = ext ? (right ? sTL + SLOT : sR + SLOT) : tp;
+            const double *xr = ext ? (right ? sPB : sR) : leaf0 ? tp : tp + SLOT;
+            const double *xs = ext ? (right ? sPS : sR + 2 * SLOT) : leaf0 ? tp : tp + 2 * SLOT;
+            const double *yl = extl ? sPB : leaf0 ? sR + SLOT : sR;
+            const double *yr = extl ? sTR + SLOT : sR + SLOT;
+            const double *ys = extl ? sPS : leaf0 ? sR + SLOT : sR + 2 * SLOT;
             double v0 = 0., v1 = 0., v2 = 0., v3 = 0., v4 = 0., v5 = 0.;
-            double ps[NR];
+            double ps[NR], pl[NR];
 #pragma unroll
             for (int r = 0; r < NR; ++r) {
-                ps[r] = T1ps[r] + Rps[r];
-                const double vT1pl = var[r] * T1pl[r], vp = var[r] * p[r];
-                const double ps1 = T1ps[r] + Rpl[r], ps2 = T1pr[r] + Rps[r];
-                v0 = fma(ps[r], vT1pl, v0); v1 = fma(ps[r], vp, v1);
-                v2 = fma(ps1, vT1pl, v2); v3 = fma(ps1, var[r] * Rpl[r], v3);
-                v4 = fma(ps2, var[r] * T1pr[r], v4); v5 = fma(ps2, vp, v5);
+                const int o = r * 32 + lane;
+                const double xpl = xl[o], xpr = xr[o], xps = xs[o], ypl = yl[o], ypr = yr[o], yps = ys[o];
+                ps[r] = xps + yps;
+                pl[r] = xpl;
+                // nuts.py:86-98: Tree.extend updates self.p_sum in place BEFORE p_sum1 / p_sum2 are formed, so the whole
+                // tree's p_sum entering them is already the total (see the oracle, bf_oracle.c tree_extend)
+                const double xq = (ext && right) ? ps[r] : xps, yq = (ext && !right) ? ps[r] : yps;
+                const double vxl = var[r] * xpl, vyr = var[r] * ypr;
+                const double ps1 = xq + ypl, ps2 = xpr + yq;
+                v0 = fma(ps[r], vxl, v0); v1 = fma(ps[r], vyr, v1);
+                v2 = fma(ps1, vxl, v2); v3 = fma(ps1, var[r] * ypl, v3);
+                v4 = fma(ps2, var[r] * xpr, v4); v5 = fma(ps2, vyr, v5);
             }
             const bool turning = quad_any_nonpos6(v0, v1, v2, v3, v4, v5, lane);
             const double um = uni(t);
-            if (need) {
+            if (go) {
                 t += 1;
-                WT T1W; T1W.m = ssc[lv * 8]; T1W.k = (int)ssc[(10 + lv) * 8];
-                const int T1slot = (int)ssc[(40 + lv) * 8];
-                const WT tot = wt_add(T1W, RW);
-                if (!wt_select(um, tot, RW)) {               // keep tree1's proposal (nuts.py:164-167)
-                    freemask |= 1u << Rslot;
-                    Rslot = T1slot; REp = ssc[(20 + lv) * 8]; Rlpp = ssc[(30 + lv) * 8];
-                } else {
-                    freemask |= 1u << T1slot;
+                WT TW; double TE, Tlp; int Tslot;
+                if (ext) { TW = Wtree; TE = prop_E; Tlp = prop_lp; Tslot = prop_slot; }
+                else {
+                    TW.m = ssc[lvl * 8]; TW.k = (int)ssc[(10 + lvl) * 8];
+                    TE = ssc[(20 + lvl) * 8]; Tlp = ssc[(30 + lvl) * 8]; Tslot = (int)ssc[(40 + lvl) * 8];
                 }
-#pragma unroll
-                for (int r = 0; r < NR; ++r) { Rpl[r] = T1pl[r]; Rps[r] = ps[r]; }
-                RW = tot;
+                const WT tot = wt_add(TW, RW);
+                const bool rwin = wt_select(um, ext ? TW : tot, RW);          // R's proposal wins
+                freemask |= 1u << (rwin ? Tslot : Rslot);
+                const int wslot = rwin ? Rslot : Tslot;
+                const double wE = rwin ? REp : TE, wlp = rwin ? Rlpp : Tlp;
+                if (ext) { Wtree = tot; prop_slot = wslot; prop_E = wE; prop_lp = wlp; }
+                else { RW = tot; Rslot = wslot; REp = wE; Rlpp = wlp; }
+                double *dps = ext ? sPS : sR + 2 * SLOT;
+                VST(dps, ps)
+                VST(sR, pl)                               // R's new left end (after the extend R is dead)
                 if (turning) turn = true;
-                lvl++;
+                if (ext) mq = 3;
+                else { lvl++; mq = (!turn && ((ileaf >> lvl) & 1)) ? 0 : 1; }
             }
-            need = need && !turn && ((ileaf >> lvl) & 1);
         }
         TICK(4)
-        const bool fin = live && (div_now || turn || (ileaf + 1 == (1 << depth)));
+        // section: push
+        // ---- push R onto the stack at level lvl ----
         const bool push = live && !fin;
         if (__any_sync(BFB_FULL, push)) {
-            const int lv = push ? lvl : 1;
-            if (__any_sync(BFB_FULL, lv > LS)) {
-                double *sp = stack_ptr(lv);
-                if (push) { VST(sp, Rpl) VST(sp + SLOT, p) VST(sp + 2 * SLOT, Rps) }
-            } else {
-                double *sp = sST + (lv - 1) * 3 * SLOT;
-                if (push) { VST(sp, Rpl) VST(sp + SLOT, p) VST(sp + 2 * SLOT, Rps) }
-            }
+            double *sp = stack_ptr(push ? lvl : 1);
             if (push) {
+                double a[NR], b[NR];
+                VLD(a, sR) VLD(b, sR + 2 * SLOT)
+                VST(sp, a) VST(sp + SLOT, p) VST(sp + 2 * SLOT, b)
                 ssc[lvl * 8] = RW.m; ssc[(10 + lvl) * 8] = (double)RW.k; ssc[(20 + lvl) * 8] = REp; ssc[(30 + lvl) * 8] = Rlpp;
                 ssc[(40 + lvl) * 8] = (double)Rslot;
                 ileaf += 1;
             }
         }
         TICK(5)
-        // ================= end of a doubling: Tree.extend, nuts.py:45-103 =================
-        if (__any_sync(BFB_FULL, fin)) {
-            const double ue = uni(t);
-            const bool right = step > 0.;
-            if (fin) {
-                double *dst = right ? sTR : sTL;
-                VST(dst, q) VST(dst + SLOT, p) VST(dst + 2 * SLOT, g)
-                depth += 1;
-            }
-            const bool ok = fin && !div_now && !turn;
-            double PS[NR], PB[NR], TLp[NR], TRp[NR];
-            VLD(PS, sPS) VLD(PB, sPB) VLD(TLp, sTL + SLOT) VLD(TRp, sTR + SLOT)
-            double v0 = 0., v1 = 0., v2 = 0., v3 = 0., v4 = 0., v5 = 0.;
-#pragma unroll
-            for (int r = 0; r < NR; ++r) {
-                PS[r] += Rps[r];
-                const double vp = var[r] * p[r], vRpl = var[r] * Rpl[r], vPB = var[r] * PB[r];
-                const double vTL = var[r] * TLp[r], vTR = var[r] * TRp[r];
-                v0 = fma(PS[r], vTL, v0); v1 = fma(PS[r], vTR, v1);
-                // nuts.py:86-98: self.p_sum is updated in place BEFORE p_sum1 / p_sum2 are formed, so the
-                // "old tree" p_sum entering them is already the total (see the oracle, bf_oracle.c tree_extend)
-                if (right) {
-                    const double ps1 = PS[r] + Rpl[r], ps2 = PB[r] + Rps[r];
-                    v2 = fma(ps1, vTL, v2); v3 = fma(ps1, vRpl, v3); v4 = fma(ps2, vPB, v4); v5 = fma(ps2, vp, v5);
-                } else {
-                    const double ps1 = Rps[r] + PB[r], ps2 = Rpl[r] + PS[r];
-                    v2 = fma(ps1, vp, v2); v3 = fma(ps1, vPB, v3); v4 = fma(ps2, vRpl, v4); v5 = fma(ps2, vTR, v5);
-                }
-            }
-            const bool turning = quad_any_nonpos6(v0, v1, v2, v3, v4, v5, lane);
-            if (ok) {
-                t += 1;
-                const WT tot = wt_add(Wtree, RW);
-                if (wt_select(ue, Wtree, RW)) {               // nuts.py:81-83 biased progressive: log(u) < size2 - size1
-                    freemask |= 1u << prop_slot;
-                    prop_slot = Rslot; prop_E = REp; prop_lp = Rlpp;
-                } else {
-                    freemask |= 1u << Rslot;
-                }
-                Wtree = tot;
-                VST(sPS, PS)
-                if (turning) turn = true;
-            }
-            if (fin) {
-                const bool iter_end = div_now || turn || (depth >= cfg.max_treedepth);
-                bnd = iter_end;
-                ns_dbl = !iter_end;
-            }
+        // section: extend
+        // ================= end of a doubling: the rest of Tree.extend, nuts.py:45-103 =================
+        if (fin) {
+            double *dst = right ? sTR : sTL;
+            VST(dst, q) VST(dst + SLOT, p) VST(dst + 2 * SLOT, g)
+            depth += 1;
+            const bool iter_end = div_now || turn || (depth >= cfg.max_treedepth);
+            bnd = iter_end;
+            ns_dbl = !iter_end;
         }
         TICK(6)
     }
 
+    // section: persist
     // ---- persist chain state ----
-    if (exists && st.status[c] == 0) {
+    // the unit's group and chunk are recomputed rather than kept live across the loop (the register file is full)
+    const int group_e = (int)((gpr - gprop) / (BFB_NSLOT * 2 * SLOT)), chunk_e = (it_hi - 1) / chunk_iters;
+    if (gi < cpg && (int64_t)group_e * cpg + gi < st.C && st.status[c] == 0) {
 #pragma unroll
         for (int r = 0; r < NR; ++r) {
             const int j = 4 * r + lg;
@@ -571,11 +538,11 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
         for (int k_ = 0; k_ < 7; ++k_) { atomicAdd(st.tree_total + 4 + k_, (unsigned long long)tacc[k_]); tsum += tacc[k_]; }
         atomicAdd(st.tree_total + 11, (unsigned long long)(clock64() - t_unit0 - tsum));
 #endif
-        qv[2 + group] = chunk + 1;
-        if ((chunk + 1) * chunk_iters < out.n_iter) {
+        qv[2 + group_e] = chunk_e + 1;
+        if ((chunk_e + 1) * chunk_iters < out.n_iter) {
             const int ti = atomicAdd(queue + 1, 1);
             __threadfence();
-            ring[ti] = group;
+            ring[ti] = group_e;
         }
     }
     }   // unit loop
@@ -910,14 +877,15 @@ static int launch_dmma(bfb_context *h, const bfb_run_out &o, int n_iter, int cpg
     const int64_t C = h->cs.C;
     const int n_groups = (int)((C + cpg - 1) / cpg);
     // one persistent block of W warps per SM (W = 4: one warp per scheduler, 4096 chains = 512 warps on 592 schedulers;
-    // W = 8 when there are more groups than that); the first LS levels of the tree stack live in shared memory, deeper
-    // (rarely touched) levels in an L2-resident buffer
+    // W = 8 when there are more groups than that); level 0 of the tree stack (the current subtree) and the next LS levels
+    // live in shared memory, deeper (rarely touched) levels in an L2-resident buffer.  LS = 0 needs as much shared memory
+    // as one stack level did when level 0 stayed in registers, so the same models fit.
     const size_t fixed = sizeof(double) * (SH::frag_doubles(W) + SH::MSM_DOUBLES + (SH::C3 ? dmma_c3_doubles(NR, h->dm.c3_kt, W) : 0));
-    if (fixed + sizeof(double) * W * warp_smem_doubles(NR, 1) > (size_t)(227 * 1024)) return 1;      // does not fit: generic kernel
+    if (fixed + sizeof(double) * W * warp_smem_doubles(NR, 0) > (size_t)(227 * 1024)) return 1;      // does not fit: generic kernel
     const size_t budget = (size_t)(227 * 1024) - 1024 - fixed;
     int LS = L;
-    while (LS > 1 && sizeof(double) * W * warp_smem_doubles(NR, LS) > budget) --LS;
-    if (const char *e = getenv("BFB200_STACK_LEVELS_SMEM")) { int v = atoi(e); if (v >= 1 && v <= L) LS = v; }
+    while (LS > 0 && sizeof(double) * W * warp_smem_doubles(NR, LS) > budget) --LS;
+    if (const char *e = getenv("BFB200_STACK_LEVELS_SMEM")) { int v = atoi(e); if (v >= 0 && v <= L) LS = v; }
     const size_t smem = fixed + sizeof(double) * W * warp_smem_doubles(NR, LS);
     BFB_REQUIRE(smem <= 227 * 1024, BFB_ERR_ARG, "sampler needs %zu bytes of shared memory per block (> 227 KB)", smem);
     BFB_CUDA(cudaFuncSetAttribute(nuts_dmma_kernel<NR, MV, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
