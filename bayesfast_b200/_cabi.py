@@ -113,6 +113,7 @@ def lib():
                     ('bfb_fit_max_beta', [C.c_void_p, C.c_void_p, C.c_int64, _dp, _dp, C.POINTER(C.c_double), C.c_void_p, C.c_int], C.c_int),
                     ('bfb_chain_diagnostics', [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int,
                                                C.c_void_p], C.c_int),
+                    ('bfb_norminv_fill', [C.c_void_p, _dp, C.c_int64, _dp, _dp], C.c_int),
                     ):
                 if hasattr(L, name):
                     f = getattr(L, name)
@@ -421,6 +422,12 @@ class Handle:
         u, z = np.empty(count), np.empty(count)
         check(self._L.bfb_rng_fill(self._h, int(seed), int(chain), int(t0), int(count), _d(u), _d(z)))
         return u, z
+
+    def norminv_fill(self, p):
+        p = np.ascontiguousarray(p, dtype=np.float64)
+        z, z_ref = np.empty_like(p), np.empty_like(p)
+        check(self._L.bfb_norminv_fill(self._h, _d(p), p.size, _d(z), _d(z_ref)))
+        return z, z_ref
 
     def fp64_peak(self, kind=0):
         v = C.c_double(0)

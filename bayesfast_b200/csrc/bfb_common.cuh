@@ -10,6 +10,8 @@
 #define BFB_NSTAGE 3    // device staging buffers of the host-output pipeline of bfb_sampler_run
 #define BFB_WARP 32
 #define BFB_FULL 0xffffffffu
+// ChainState::tree_total: [0] leapfrogs in trees, [1..19] round / section counters and cycle sums of the timing builds
+#define BFB_TREE_TOTAL_LEN 20
 
 void bfb_set_error(const char *fmt, ...);
 
@@ -118,7 +120,7 @@ struct ChainState {
     int64_t *t_draw;                                 // [C]
     int64_t *iter;                                   // [C] iterations done
     int32_t *status;                                 // [C]
-    unsigned long long *tree_total;                  // [4]: leapfrogs in trees; debug counters of the multi-chain kernels
+    unsigned long long *tree_total;                  // [BFB_TREE_TOTAL_LEN]: leapfrogs in trees; debug counters of the multi-chain kernels
     // dense mass matrix (bfb_sampler_init_dense; generic kernel only): [C][n][np], transposed XT[k][j] = X[j][k]
     double *covT, *cholT, *cholW, *fgcT, *bgcT;      // covariance, its Cholesky factor (+ work copy), Welford fore/background
     int32_t *chol_error;                             // [C]

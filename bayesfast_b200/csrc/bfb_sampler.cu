@@ -625,7 +625,7 @@ static int sampler_init_common(bfb_handle h, const bfb_sampler_cfg *cfg, int64_t
     const bool reuse = !h->chain_allocs.empty() && h->alloc_C == C && h->alloc_np == np && !h->chain_snapshot.empty();
     if (reuse) {
         for (auto &a : state_arrays(s)) BFB_CUDA(cudaMemsetAsync(a.first, 0, a.second, h->stream));
-        BFB_CUDA(cudaMemsetAsync(s.tree_total, 0, 16 * sizeof(unsigned long long), h->stream));
+        BFB_CUDA(cudaMemsetAsync(s.tree_total, 0, BFB_TREE_TOTAL_LEN * sizeof(unsigned long long), h->stream));
     } else {
         bfb_free_list(h->chain_allocs);
         h->chain_snapshot.clear();
@@ -639,7 +639,7 @@ static int sampler_init_common(bfb_handle h, const bfb_sampler_cfg *cfg, int64_t
             (rc = dalloc(h, &s.hbar, C)) || (rc = dalloc(h, &s.mu_da, C)) || (rc = dalloc(h, &s.count, C)) ||
             (rc = dalloc(h, &s.n_samples, C)) || (rc = dalloc(h, &s.previous_update, C)) ||
             (rc = dalloc(h, &s.adapt_window, C)) || (rc = dalloc(h, &s.t_draw, C)) || (rc = dalloc(h, &s.iter, C)) ||
-            (rc = dalloc(h, &s.status, C)) || (rc = dalloc(h, &s.tree_total, 16)))
+            (rc = dalloc(h, &s.status, C)) || (rc = dalloc(h, &s.tree_total, BFB_TREE_TOTAL_LEN)))
             return rc;
         for (auto &a : state_arrays(s)) {
             void *p = nullptr;
@@ -1095,7 +1095,7 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
     const int n = h->n;
     void *const user[11] = {out->samples, out->logp, out->energy, out->mean_tree_accept, out->step_size, out->step_size_bar,
                             out->energy_change, out->max_energy_change, out->tree_depth, out->tree_size, out->diverging};
-    BFB_CUDA(cudaMemsetAsync(h->cs.tree_total, 0, 16 * sizeof(unsigned long long), h->stream));
+    BFB_CUDA(cudaMemsetAsync(h->cs.tree_total, 0, BFB_TREE_TOTAL_LEN * sizeof(unsigned long long), h->stream));
     unsigned long long tt = 0;
     const bfb_run_out none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     BFB_CUDA(cudaEventRecord(h->ev0, h->stream));
@@ -1267,7 +1267,7 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
     BFB_CUDA(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
     if (total_tree_size) *total_tree_size = (int64_t)tt;
     if (getenv("BFB200_DEBUG")) {
-        unsigned long long dbg[16];
+        unsigned long long dbg[BFB_TREE_TOTAL_LEN];
         BFB_CUDA(cudaMemcpy(dbg, h->cs.tree_total, sizeof(dbg), cudaMemcpyDeviceToHost));
         fprintf(stderr, "[bfb200] leaves %llu warp-rounds %llu merge-passes %llu iter-end-sections %llu  ms %.3f\n", dbg[0], dbg[1], dbg[2], dbg[3], h->last_ms);
         if (dbg[1] && h->last_path == 3)
@@ -1279,9 +1279,15 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
                     (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
                     (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1], dbg[12],
                     (double)dbg[13] / (dbg[12] ? dbg[12] : 1), (double)dbg[14] / (dbg[12] ? dbg[12] : 1), (double)dbg[15] / (dbg[12] ? dbg[12] : 1));
-        else if (dbg[1]) fprintf(stderr, "[bfb200] cycles per warp-round: boundary %.0f rng+dbl %.0f (unused) %.0f leaves %.0f merge-loop %.0f push %.0f extend %.0f | unit setup+teardown per round %.0f\n",
-                            (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
-                            (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1]);
+        else if (dbg[1]) {
+            const double bnd = (double)(dbg[4] + dbg[16] + dbg[17] + dbg[18] + dbg[19]);
+            fprintf(stderr, "[bfb200] cycles per warp-round: boundary %.0f rng+dbl %.0f (unused) %.0f leaves %.0f merge-loop %.0f push %.0f extend %.0f | unit setup+teardown per round %.0f\n",
+                    bnd / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
+                    (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1]);
+            fprintf(stderr, "[bfb200] boundary cycles per warp-round: statistics %.0f lane-per-dimension %.0f progress-report %.0f new-state %.0f rest %.0f | rounds with a boundary %.3f\n",
+                    (double)dbg[16] / dbg[1], (double)dbg[17] / dbg[1], (double)dbg[18] / dbg[1], (double)dbg[19] / dbg[1],
+                    (double)dbg[4] / dbg[1], (double)dbg[3] / dbg[1]);
+        }
     }
     return BFB_OK;
 }

@@ -122,7 +122,8 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
     double e_step = exp(log_step), e_bar = exp(log_bar);    // refreshed only when dual averaging moves them
     int status = exists ? st.status[c] : 9;
     unsigned tree_total = 0, dbg_rounds = 0, dbg_merges = 0, dbg_iend = 0; (void)dbg_rounds; (void)dbg_merges; (void)dbg_iend;
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64(); (void)tacc; (void)tlast;
+    // tacc: 0..6 the sections of a round (0: the boundary outside its parts), 7 the loop head, 8..11 the boundary's parts
+    long long tacc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64(); (void)tacc; (void)tlast;
     bool done = (status != 0) || it_lo >= it_hi;
     int it = it_lo;
     // progress reports (host outputs of a single launch, bfb_sampler_run_ex): every chain counts itself in when it has finished a
@@ -143,8 +144,9 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
     bool bnd = !done, fresh = true, ns_dbl = false;
     // the current subtree R (left-end p, right-end p, p_sum) is the level-0 stack entry
     double *sR = sST;
-    // scratch vectors of the boundary section alias the (then empty) level-0 stack entry
-    double *sP0 = sST, *sVAR = sST + SLOT, *sQN = sST + 2 * SLOT;
+    // scratch vectors of the boundary section alias the (then empty) level-0 stack entry: the next state's position,
+    // gradient and metric, staged by the chain's quad for the lane-per-dimension pass
+    double *sGX = sST, *sVAR = sST + SLOT, *sQN = sST + 2 * SLOT;
 
     // stack entry of level lvl: levels 0..LS in shared memory, deeper ones in the L2-resident buffer
     auto stack_ptr = [&](int lvl) -> double * {
@@ -161,12 +163,17 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
             const bool endp = bnd && !fresh;
             const bool warm_old = (it0 + it) < cfg.n_warmup;            // of the iteration that ends
             const size_t orow = (size_t)c * out.n_iter + it;
-            // the accepted proposal (position, gradient) comes from the L2-resident pool: issue the loads first
+            // the accepted proposal (position, gradient) comes from the L2-resident pool: issue the loads first.  A fresh
+            // chain's starting point becomes the accepted proposal in slot 0 of the pool, so every chain's next state is read
+            // from there
+            if (fresh && bnd) { VST(gpr, q) VST(gpr + SLOT, g) }
             double qn[NR], gx[NR];
             {
                 const double *slot = gpr + (size_t)(endp ? prop_slot : 0) * 2 * SLOT;
                 VLD(qn, slot) VLD(gx, slot + SLOT)
             }
+            TICK(0)
+            // section: boundary statistics
             // ---- (1) per chain (its quad), predicated: accept statistic, dual averaging, statistics ----
             const double accept_stat = acc_sum / (double)(n_prop > 0 ? n_prop : 1);
             if (__any_sync(BFB_FULL, endp && warm_old && cfg.adapt_step_size)) {      // step_size.py:31-45
@@ -198,10 +205,13 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
                 it += 1;
                 if (it >= it_hi) done = true;
             }
-            if (bnd) { VST(sVAR, var) VST(sQN, qn) }
+            if (bnd) { VST(sQN, qn) VST(sGX, gx) VST(sVAR, var) }
             __syncwarp();
+            TICK(8)
+            // section: boundary lane per dimension
             // ---- (2) cooperative, lane j = dimension j, one chain at a time: new sample out, windowed Welford
-            //      metric (metrics.py:186-211, 333-371), momentum draw (metrics.py:83-86) ----
+            //      metric (metrics.py:186-211, 333-371), momentum draw (metrics.py:83-86), and the two ends and p_sum
+            //      of the new tree (Tree.__init__): position, momentum and gradient of the new state ----
             unsigned mask = __ballot_sync(BFB_FULL, bnd);
 #pragma unroll 1
             while (mask) {
@@ -246,10 +256,17 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
                 if (!(fl & 2)) {
                     double p0j = 0.;
                     if (j < n) p0j = draw_normal_ni(seed, (uint64_t)(cfg.chain0 + c_s), (uint64_t)(t_s + j)) / sqrt(sVAR[e]);
-                    if (j < 4 * NR) sP0[e] = p0j;
+                    if (j < 4 * NR) {
+                        const double qj = sQN[e], gj = sGX[e];
+                        sTL[e] = qj; sTL[SLOT + e] = p0j; sTL[2 * SLOT + e] = gj;
+                        sTR[e] = qj; sTR[SLOT + e] = p0j; sTR[2 * SLOT + e] = gj;
+                        sPS[e] = p0j;
+                    }
                 }
             }
             __syncwarp();
+            TICK(9)
+            // section: boundary progress report
             {
                 const bool hit = endp && it == next_rep;          // this chain's records of report chunk (it - 1) / rep_it are written
                 if (__any_sync(BFB_FULL, hit)) {
@@ -269,37 +286,30 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
                     }
                 }
             }
+            TICK(10)
+            // section: boundary new state
             // ---- (3) per chain, predicated: the new state and the empty tree ----
             double p0[NR], part = 0.;
-            {
-                double vn[NR];
-                VLD(vn, sVAR) VLD(p0, sP0)
-                if (bnd) {
-#pragma unroll
-                    for (int r = 0; r < NR; ++r) { if (!fresh) { q[r] = qn[r]; g[r] = gx[r]; } var[r] = vn[r]; }
-                }
-            }
+            VLD(p0, sTL + SLOT)
+            if (bnd) { VLD(q, sQN) VLD(g, sGX) VLD(var, sVAR) }
 #pragma unroll
             for (int r = 0; r < NR; ++r) part = fma(p0[r], var[r] * p0[r], part);
             const double ke = qsum(part);
             const bool warm_new = (it0 + it) < cfg.n_warmup;
             const bool startp = bnd && !done;
-            __syncwarp();                                     // sP0 / sVAR alias the level-0 stack entry: reads before writes
             if (startp) {
                 t += n;
                 E0 = 0.5 * ke - logp_q;
                 if (!isfinite(E0)) { status = 2; done = true; }
                 step = warm_new ? e_step : e_bar;
-                VST(sTL, q) VST(sTL + SLOT, p0) VST(sTL + 2 * SLOT, g)
-                VST(sTR, q) VST(sTR + SLOT, p0) VST(sTR + 2 * SLOT, g)
-                VST(sPS, p0)
-                if (fresh) { VST(gpr, q) VST(gpr + SLOT, g) prop_slot = 0; }    // starting point = slot of the accepted proposal
+                if (fresh) prop_slot = 0;
                 freemask = ((1u << BFB_NSLOT) - 1u) & ~(1u << prop_slot);
                 prop_E = E0; prop_lp = logp_q; Wtree.m = 1.; Wtree.k = 0; acc_sum = 0.; maxdE = 0.;
                 depth = 0; n_prop = 0; diverging = 0;
                 ns_dbl = !done;
             }
             bnd = false; fresh = false;
+            TICK(11)
             if (!__any_sync(BFB_FULL, !done)) break;
         }
         const bool live = !done;
@@ -536,6 +546,7 @@ __global__ void __launch_bounds__(32 * W, 1) nuts_dmma_kernel(DevModel M, bfb_sa
         atomicAdd(st.tree_total + 3, (unsigned long long)dbg_iend);
         long long tsum = 0;
         for (int k_ = 0; k_ < 7; ++k_) { atomicAdd(st.tree_total + 4 + k_, (unsigned long long)tacc[k_]); tsum += tacc[k_]; }
+        for (int k_ = 8; k_ < 12; ++k_) { atomicAdd(st.tree_total + 8 + k_, (unsigned long long)tacc[k_]); tsum += tacc[k_]; }
         atomicAdd(st.tree_total + 11, (unsigned long long)(clock64() - t_unit0 - tsum));
 #endif
         qv[2 + group_e] = chunk_e + 1;
@@ -1011,5 +1022,33 @@ int bfb_launch_nuts_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
     BFB_CASE(4, 5) BFB_CASE(4, 7) BFB_CASE(7, 5) BFB_CASE(7, 7)          // with cubic-3 configs (n <= 28)
 #undef BFB_CASE
     return 1;
+}
+#endif
+
+#ifndef BFB_DMMA_PART_HEADLINE
+__global__ void norminv_fill_kernel(const double *p, int64_t count, double *z, double *z_ref)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    z[i] = bfb_norminv_small(p[i]);
+    z_ref[i] = bfb_norminv(p[i]);
+}
+
+extern "C" int bfb_norminv_fill(bfb_handle h, const double *p, int64_t count, double *z, double *z_ref)
+{
+    BFB_REQUIRE(h && p && z && z_ref && count >= 0, BFB_ERR_ARG, "bfb_norminv_fill: bad arguments");
+    if (count == 0) return BFB_OK;
+    BFB_CUDA(cudaSetDevice(h->device));
+    double *dp;
+    BFB_CUDA(cudaMalloc(&dp, sizeof(double) * 3 * count));
+    BFB_CUDA(cudaMemcpyAsync(dp, p, sizeof(double) * count, cudaMemcpyHostToDevice, h->stream));
+    norminv_fill_kernel<<<(unsigned)((count + 255) / 256), 256, 0, h->stream>>>(dp, count, dp + count, dp + 2 * count);
+    h->launches++;
+    BFB_CUDA(cudaGetLastError());
+    BFB_CUDA(cudaMemcpyAsync(z, dp + count, sizeof(double) * count, cudaMemcpyDeviceToHost, h->stream));
+    BFB_CUDA(cudaMemcpyAsync(z_ref, dp + 2 * count, sizeof(double) * count, cudaMemcpyDeviceToHost, h->stream));
+    BFB_CUDA(cudaStreamSynchronize(h->stream));
+    cudaFree(dp);
+    return BFB_OK;
 }
 #endif

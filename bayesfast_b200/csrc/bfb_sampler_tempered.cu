@@ -504,7 +504,7 @@ extern "C" int bfb_tsampler_run(bfb_handle h, int sampler, int32_t n_iter, const
     od.o.max_energy_change = (double *)dev[7];
     od.o.tree_depth = (int32_t *)dev[8]; od.o.tree_size = (int32_t *)dev[9]; od.o.diverging = (int32_t *)dev[10];
     od.u = (double *)dev[11]; od.weight = (double *)dev[12];
-    cudaError_t e = cudaMemsetAsync(h->cs.tree_total, 0, 16 * sizeof(unsigned long long), h->stream);
+    cudaError_t e = cudaMemsetAsync(h->cs.tree_total, 0, BFB_TREE_TOTAL_LEN * sizeof(unsigned long long), h->stream);
     int rc = BFB_OK;
     if (e == cudaSuccess) {
         cudaEventRecord(h->ev0, h->stream);

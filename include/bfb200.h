@@ -253,6 +253,9 @@ int64_t bfb_launch_count(bfb_handle h);
 /* draws t0..t0+count-1 of the stream (seed, chain) computed ON THE DEVICE: u (uniform view) and z (normal
  * view).  Host pointers.  Used by the parity tests to teacher-force the oracle. */
 int bfb_rng_fill(bfb_handle h, uint64_t seed, uint64_t chain, uint64_t t0, int64_t count, double *u, double *z);
+/* Phi^-1 of count probabilities p in (0, 1) computed ON THE DEVICE, twice: z by the restatement the tensor-core samplers
+ * draw their momenta with, z_ref by bfb_norminv of bfb_rng.h.  Host pointers.  The two must agree bit for bit. */
+int bfb_norminv_fill(bfb_handle h, const double *p, int64_t count, double *z, double *z_ref);
 
 /* FP64 peak microbenchmarks for the roofline denominator (MEASURED_PEAKS.json has no FP64 entry):
  * kind 0 = DFMA, 1 = DMMA m8n8k4, 2 = both interleaved.  Returns TFLOP/s. */

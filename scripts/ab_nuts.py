@@ -87,7 +87,6 @@ def main():
                 for ln in p.stderr.splitlines():
                     if 'cycles per' in ln:
                         print('%s round %d: %s' % (tag, rnd, ln), flush=True)
-                        break
     med = {k: float(np.median(v)) for k, v in res.items()}
     print(json.dumps(dict(gpu=gpu, rounds=a.rounds, launches_per_process=a.launches,
                           old_ms=dict(median=med['old'], min=min(res['old']), max=max(res['old'])),
