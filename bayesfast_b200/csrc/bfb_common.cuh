@@ -163,7 +163,7 @@ struct bfb_context {
     size_t stage_len[BFB_NSTAGE];
     int *queue;                // work queue of the multi-chain kernel
     size_t queue_len;
-    int last_path;             // kernel family of the last sampler launch: 0 generic, 1 FMA multi-chain, 2 tensor core
+    int last_path;             // kernel family of the last sampler launch: 0 generic, 2 dmma, 3 team, 4 pair (bfb_sampler.cu: FAM_*)
     int64_t iters_done;        // iterations completed by every chain since bfb_sampler_init / reset
     double *lik_tab;           // operand table of the tensor-core likelihood evaluator (bfb_lik_dmma.cu), or null
     int lik_nr;

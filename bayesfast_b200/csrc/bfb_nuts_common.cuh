@@ -1,7 +1,8 @@
 // bfb_nuts_common.cuh -- pieces shared by the multi-chain-per-warp NUTS kernels (bfb_sampler_dmma.cu, bfb_sampler_team.cu,
-// bfb_sampler_pair.cu): linear-domain multinomial weights, the run-output descriptor and the work-queue initialiser.
+// bfb_sampler_pair.cu): linear-domain multinomial weights, the run-output descriptor, the work queue and the deep tree stack.
 #pragma once
 #include "bfb_common.cuh"
+#include <cstdlib>
 
 struct RunOutDevF {
     bfb_run_out o;
@@ -53,4 +54,44 @@ static __global__ void queue_init_kernel(int *queue, int n_groups, int n_units, 
     if (i == 0) { queue[0] = head0; queue[1] = n_groups; }
     if (i < n_groups) queue[2 + i] = 0;
     if (i < n_units) queue[2 + n_groups + i] = (i < n_groups) ? i : -1;
+}
+
+// Work queue of a persistent sampler kernel for n_iter iterations of n_groups groups: units of chunk_iters iterations
+// (default_chunks per group, at least 16 iterations each, BFB200_CHUNK_ITERS overrides), h->queue grown to hold the queue and
+// `extra` ints behind it, and the initialiser launched on h->stream.
+static inline int queue_setup(bfb_context *h, int n_groups, int n_iter, int default_chunks, int head0, size_t extra,
+                              int &chunk_iters, int &n_units)
+{
+    chunk_iters = (n_iter + default_chunks - 1) / default_chunks;
+    if (chunk_iters < 16) chunk_iters = n_iter < 16 ? n_iter : 16;
+    if (const char *e = getenv("BFB200_CHUNK_ITERS")) { int v = atoi(e); if (v >= 1) chunk_iters = v; }
+    const int n_chunks = (n_iter + chunk_iters - 1) / chunk_iters;
+    const int64_t n_units64 = (int64_t)n_groups * n_chunks;
+    BFB_REQUIRE(n_units64 < (1ll << 31), BFB_ERR_ARG, "too many work units");
+    n_units = (int)n_units64;
+    const size_t qlen = 2 + (size_t)n_groups + (size_t)n_units64 + extra;
+    if (qlen > h->queue_len) {
+        if (h->queue) cudaFree(h->queue);
+        h->queue = nullptr; h->queue_len = 0;
+        BFB_CUDA(cudaMalloc((void **)&h->queue, sizeof(int) * qlen));
+        h->queue_len = qlen;
+    }
+    queue_init_kernel<<<(unsigned)((n_units64 + 255) / 256), 256, 0, h->stream>>>(h->queue, n_groups, n_units, head0);
+    h->launches++;
+    return BFB_OK;
+}
+
+// h->gstack of a tree-building kernel, grown on demand: per group the stack levels LS + 1 .. L - 1 that do not fit in shared
+// memory (3 vectors of `slot` doubles each) at h->gstack, then per group the proposal pool (n_prop x 2 vectors) at *gprop
+static inline int gstack_reserve(bfb_context *h, int n_groups, int L, int LS, int slot, int n_prop, double **gprop)
+{
+    const size_t deep = (size_t)(L - 1 > LS ? L - 1 - LS : 0) * 3 * slot, prop = (size_t)n_prop * 2 * slot;
+    if ((deep + prop) * (size_t)n_groups > h->gstack_len) {
+        if (h->gstack) cudaFree(h->gstack);
+        h->gstack = nullptr; h->gstack_len = 0;
+        BFB_CUDA(cudaMalloc((void **)&h->gstack, sizeof(double) * (deep + prop) * (size_t)n_groups));
+        h->gstack_len = (deep + prop) * (size_t)n_groups;
+    }
+    *gprop = h->gstack + deep * (size_t)n_groups;
+    return BFB_OK;
 }

@@ -18,6 +18,7 @@
 #include <cstdio>
 #include <cstdlib>
 
+// the kernel of the family select_family chose for the model: 0 on launch, 1 when its shared memory does not fit, < 0 on error
 int bfb_launch_nuts_dmma(bfb_context *h, const bfb_run_out &o, int n_iter);   // bfb_sampler_dmma.cu
 int bfb_launch_hmc_dmma(bfb_context *h, const bfb_run_out &o, int n_iter);    // bfb_sampler_dmma.cu
 int bfb_launch_nuts_team(bfb_context *h, const bfb_run_out &o, int n_iter);   // bfb_sampler_team.cu
@@ -809,40 +810,69 @@ static int launch_sampler(bfb_context *h, const RunOutDev &out, int wpb)
     return h->dense_metric ? launch_sampler<NPL, SAMPLER, true>(h, out, wpb) : launch_sampler<NPL, SAMPLER, false>(h, out, wpb);
 }
 
+// kernel families of the sampler, numbered as bfb_sampler_last_path reports them
+enum { FAM_GENERIC = 0, FAM_DMMA = 2, FAM_TEAM = 3, FAM_PAIR = 4 };
+static const char *const fam_name[] = {"generic", nullptr, "dmma", "team", "pair"};
+// what the family's kernels take, for the error when a pinned family cannot run the model
+static const char *const fam_needs[] = {nullptr, nullptr,
+    "n <= 32 without a prior (with cubic-3 configs: n <= 28 and cubic-2 ones), or the likelihood pipeline's tensor-core table",
+    "n <= 64 for HMC and 32 < n <= 64 for NUTS, without decay / transform / rescale / likelihood pipeline",
+    "NUTS with n <= 32, without a prior / cubic-3 configs / likelihood pipeline"};
+
+// The kernel family that runs `sampler` on the model and chains of h.  By default a dense mass matrix runs on the generic
+// warp-per-chain kernel.  NUTS runs on the team kernel for 32 < n <= 64, else on the one-warp kernel (dmma) where that takes
+// the model.  HMC runs on the team kernel for 32 < n <= 64 and up to four groups of 8 chains per SM (4736 chains on a B200:
+// 4096 chains 2.20e9 leapfrogs/s against 2.06e9 with one warp per group), above that on the one-warp kernel, which then has
+// enough warps and fewer instructions (16384 chains: 3.2e9 against 2.5e9).  Everything else runs on the generic kernel.
+// BFB200_SAMPLER = generic | dmma | team | pair pins a family for tests and profiles (*pinned); a pinned family that cannot
+// run the model is an error (< 0).
+static int select_family(bfb_context *h, int sampler, bool *pinned)
+{
+    const DevModel &M = h->dm;
+    const bool nuts = sampler == BFB_NUTS;
+    const bool team = !M.epilogue && M.tfrag && M.team_nr != 0 && !M.frag_ext && (!nuts || M.team_nr == 16) &&
+                      (!M.has_c3 || (M.team_nr == 16 && M.tfrag3 && M.has_c2));
+    const bool dmma = M.epilogue ? M.lik_tab != nullptr : M.frag_nr != 0 && (!M.has_c3 || (M.c3_kt != 0 && M.has_c2));
+    const bool pair = nuts && !M.epilogue && M.frag_nr != 0 && !M.has_c3;
+    const bool depth_ok = !nuts || h->scfg.max_treedepth <= 10;        // the tensor-core NUTS kernels keep at most 10 tree levels
+    const char *sel = getenv("BFB200_SAMPLER");
+    *pinned = sel != nullptr;
+    if (!sel) {
+        if (h->dense_metric || !depth_ok) return FAM_GENERIC;
+        if (team && (nuts || M.team_nr == 16 || (h->cs.C + 7) / 8 <= (int64_t)h->sm_count * 4)) return FAM_TEAM;
+        return dmma ? FAM_DMMA : FAM_GENERIC;
+    }
+    int fam = -1;
+    for (int f = 0; f <= FAM_PAIR; ++f)
+        if (fam_name[f] && !strcmp(sel, fam_name[f])) fam = f;
+    BFB_REQUIRE(fam >= 0, BFB_ERR_ARG, "BFB200_SAMPLER=%s: unknown kernel family (generic, dmma, team or pair)", sel);
+    if (fam == FAM_GENERIC) return fam;
+    BFB_REQUIRE(!h->dense_metric, BFB_ERR_ARG, "BFB200_SAMPLER=%s: a dense mass matrix runs on the generic kernel only", sel);
+    BFB_REQUIRE(depth_ok, BFB_ERR_ARG, "BFB200_SAMPLER=%s: the tensor-core NUTS kernels take max_treedepth <= 10", sel);
+    BFB_REQUIRE(fam == FAM_DMMA ? dmma : fam == FAM_TEAM ? team : pair, BFB_ERR_ARG,
+                "BFB200_SAMPLER=%s: the %s kernels cannot run this model; they take %s", sel, sel, fam_needs[fam]);
+    return fam;
+}
+
 // launch the kernel(s) that advance every chain by n_iter iterations, outputs (device pointers) laid out [C, n_iter(, n)]
 static int launch_run(bfb_context *h, int sampler, int n_iter, const bfb_run_out &dev_out)
 {
     RunOutDev od;
     od.n_iter = n_iter;
     od.o = dev_out;
-    int rc = BFB_OK, fast_rc = 1;
-    // NUTS kernel selection: a tensor-core family (one warp per 8-chain group by default; BFB200_SAMPLER = team | pair select the
-    // alternatives), then the generic warp-per-chain kernel (BFB200_SAMPLER = dmma | team | pair | generic pins one for tests and profiles)
-    const char *sel_ = getenv("BFB200_SAMPLER");
-    // a dense mass matrix runs on the generic kernel only
-    if (sampler == BFB_NUTS && !h->dense_metric && !getenv("BFB200_FORCE_GENERIC") && !(sel_ && !strcmp(sel_, "generic"))) {
-        fast_rc = bfb_launch_nuts_team(h, od.o, n_iter);
-        if (fast_rc == 0) h->last_path = 3;
-        if (fast_rc == 1) {
-            fast_rc = bfb_launch_nuts_pair(h, od.o, n_iter);
-            if (fast_rc == 0) h->last_path = 4;
-        }
-        if (fast_rc == 1) {
-            fast_rc = bfb_launch_nuts_dmma(h, od.o, n_iter);
-            if (fast_rc == 0) h->last_path = 2;
-        }
-    }
-    if (sampler == BFB_HMC && !h->dense_metric && !getenv("BFB200_FORCE_GENERIC") && !(sel_ && !strcmp(sel_, "generic"))) {
-        fast_rc = bfb_launch_hmc_team(h, od.o, n_iter);
-        if (fast_rc == 0) h->last_path = 3;
-        if (fast_rc == 1) {
-            fast_rc = bfb_launch_hmc_dmma(h, od.o, n_iter);
-            if (fast_rc == 0) h->last_path = 2;
-        }
-    }
-    if (fast_rc < 0) return fast_rc;
-    if (fast_rc == 0) return BFB_OK;
-    h->last_path = 0;
+    bool pinned;
+    const int fam = select_family(h, sampler, &pinned);
+    if (fam < 0) return fam;
+    int rc = 1;
+    if (fam == FAM_TEAM) rc = sampler == BFB_NUTS ? bfb_launch_nuts_team(h, od.o, n_iter) : bfb_launch_hmc_team(h, od.o, n_iter);
+    else if (fam == FAM_DMMA) rc = sampler == BFB_NUTS ? bfb_launch_nuts_dmma(h, od.o, n_iter) : bfb_launch_hmc_dmma(h, od.o, n_iter);
+    else if (fam == FAM_PAIR) rc = bfb_launch_nuts_pair(h, od.o, n_iter);
+    if (rc == 0) h->last_path = fam;
+    if (rc <= 0) return rc;
+    // the family's shared memory does not fit the model: the generic kernel runs it, unless the family was pinned
+    BFB_REQUIRE(!pinned || fam == FAM_GENERIC, BFB_ERR_ARG,
+                "BFB200_SAMPLER=%s: the kernel needs more than 227 KB of shared memory per block for this model", fam_name[fam]);
+    h->last_path = FAM_GENERIC;
     // warps per block: as many as the per-warp tree state leaves room for in shared memory (the evaluation is latency bound:
     // at n = 64 a warp needs 32 KB, and 7 resident warps per SM instead of 4 are 1.7x the throughput)
     const int npl = h->np / 32;
@@ -888,9 +918,9 @@ static int single_launch_host_outputs(bfb_context *h, int sampler, int R, void *
                                       const double **diag_P)
 {
     const DevModel &M = h->dm;
-    // only nuts_dmma_kernel reports progress: the same conditions as bfb_launch_nuts_dmma, default kernel selection
-    if (getenv("BFB200_SAMPLER") || getenv("BFB200_FORCE_GENERIC") || getenv("BFB200_CHAINS_PER_GROUP")) return 1;
-    if (M.epilogue || M.frag_nr == 0 || M.has_c3 || h->scfg.max_treedepth > 10) return 1;
+    // only nuts_dmma_kernel reports progress, and only when it runs by default with eight chains per group
+    bool pinned;
+    if (select_family(h, sampler, &pinned) != FAM_DMMA || pinned || M.epilogue || M.has_c3 || getenv("BFB200_CHAINS_PER_GROUP")) return 1;
     const int64_t C = h->cs.C;
     const int n = h->n;
     size_t rec = 0;
@@ -988,7 +1018,7 @@ static int single_launch_host_outputs(bfb_context *h, int sampler, int R, void *
         fill_to(it_end);
         return BFB_OK;
     };
-    if (h->last_path != 2 || h->progress_chunk_iters == 0) {
+    if (h->last_path != FAM_DMMA || h->progress_chunk_iters == 0) {
         // another kernel family took the launch: no progress reports, one copy after the kernel
         BFB_CUDA(cudaStreamWaitEvent(h->copy_stream, h->ev1, 0));
         if ((rc = copy_range(0, R))) return rc;
@@ -1270,11 +1300,11 @@ extern "C" int bfb_sampler_run_ex(bfb_handle h, int sampler, int32_t n_iter, con
         unsigned long long dbg[BFB_TREE_TOTAL_LEN];
         BFB_CUDA(cudaMemcpy(dbg, h->cs.tree_total, sizeof(dbg), cudaMemcpyDeviceToHost));
         fprintf(stderr, "[bfb200] leaves %llu warp-rounds %llu merge-passes %llu iter-end-sections %llu  ms %.3f\n", dbg[0], dbg[1], dbg[2], dbg[3], h->last_ms);
-        if (dbg[1] && h->last_path == 3)
+        if (dbg[1] && h->last_path == FAM_TEAM)
             fprintf(stderr, "[bfb200] team kernel, leader-warp cycles per round: apply %.0f boundary %.0f leapfrog+eval %.0f owners %.0f tasks+leaf %.0f decisions %.0f command-barrier %.0f\n",
                     (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
                     (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1]);
-        else if (dbg[1] && h->last_path == 4)
+        else if (dbg[1] && h->last_path == FAM_PAIR)
             fprintf(stderr, "[bfb200] pair kernel, tree warp cycles per round: boundary %.0f rng+dbl %.0f wait-for-leaves %.0f leaf-pair %.0f merges %.0f push %.0f extend %.0f hand-over %.0f | integrator (%llu rounds): wait-unit %.0f wait-tree %.0f compute %.0f\n",
                     (double)dbg[4] / dbg[1], (double)dbg[5] / dbg[1], (double)dbg[6] / dbg[1], (double)dbg[7] / dbg[1],
                     (double)dbg[8] / dbg[1], (double)dbg[9] / dbg[1], (double)dbg[10] / dbg[1], (double)dbg[11] / dbg[1], dbg[12],

@@ -779,26 +779,13 @@ static int launch_hmc_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
     BFB_CUDA(cudaFuncSetAttribute(hmc_dmma_kernel<NR, MV, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     RunOutDevF od;
     od.o = o; od.n_iter = n_iter;
-    int chunk_iters = (n_iter + 5) / 6;
-    if (chunk_iters < 16) chunk_iters = n_iter < 16 ? n_iter : 16;
-    if (const char *e = getenv("BFB200_CHUNK_ITERS")) { int v = atoi(e); if (v >= 1) chunk_iters = v; }
-    const int n_chunks = (n_iter + chunk_iters - 1) / chunk_iters;
-    const int64_t n_units64 = (int64_t)n_groups * n_chunks;
-    BFB_REQUIRE(n_units64 < (1ll << 31), BFB_ERR_ARG, "too many work units");
-    const size_t qlen = 2 + (size_t)n_groups + (size_t)n_units64;
-    if (qlen > h->queue_len) {
-        if (h->queue) cudaFree(h->queue);
-        h->queue = nullptr; h->queue_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->queue, sizeof(int) * qlen));
-        h->queue_len = qlen;
-    }
-    queue_init_kernel<<<(unsigned)((n_units64 + 255) / 256), 256, 0, h->stream>>>(h->queue, n_groups, (int)n_units64);
-    h->launches++;
+    int chunk_iters, n_units, rc;
+    if ((rc = queue_setup(h, n_groups, n_iter, 6, 0, 0, chunk_iters, n_units))) return rc;
     int blocks = h->sm_count;
     const int64_t want = (n_groups + W - 1) / W;
     if ((int64_t)blocks > want) blocks = (int)want;
     hmc_dmma_kernel<NR, MV, W><<<blocks, 32 * W, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, (int)h->iters_done, chunk_iters,
-                                                                   n_groups, (int)n_units64, h->queue);
+                                                                   n_groups, n_units, h->queue);
     h->launches++;
     BFB_CUDA(cudaGetLastError());
     return BFB_OK;
@@ -834,24 +821,21 @@ int bfb_launch_nuts_dmma_headline(bfb_context *h, const bfb_run_out &o, int n_it
 #ifdef BFB_DMMA_PART_HEADLINE
 int bfb_launch_hmc_dmma_headline(bfb_context *h, const bfb_run_out &o, int n_iter) { return launch_hmc_dmma_w<7, 1>(h, o, n_iter); }
 #else
-// returns 1 if this path does not apply (caller uses the generic kernel), 0 on launch, <0 on error
+// launches the HMC kernel of the model (select_family, bfb_sampler.cu, chose this family): 0 on launch, 1 when its shared memory
+// does not fit, < 0 on error
 int bfb_launch_hmc_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     const DevModel &M = h->dm;
-    if (M.epilogue) {                       // likelihood pipeline (model variant bit 3): operand streamed from L2
-        if (!M.lik_tab) return 1;
-        if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "dmma")) return 1; }
-        if (M.lik_ftab) {                 // feature form: two chained GEMMs per 8 outputs (model variant bit 4)
-            switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
-            case 8: return launch_hmc_dmma_w<4, 24>(h, o, n_iter);
-            case 14: return launch_hmc_dmma_w<7, 24>(h, o, n_iter);
-            case 16: return launch_hmc_dmma_w<8, 24>(h, o, n_iter);
-            case 9: return launch_hmc_dmma_w<4, 26>(h, o, n_iter);
-            case 15: return launch_hmc_dmma_w<7, 26>(h, o, n_iter);
-            case 17: return launch_hmc_dmma_w<8, 26>(h, o, n_iter);
-            }
-            return 1;
+    if (M.epilogue && M.lik_ftab) {         // likelihood pipeline (model variant bit 3), feature form: two chained GEMMs per 8 outputs (bit 4)
+        switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
+        case 8: return launch_hmc_dmma_w<4, 24>(h, o, n_iter);
+        case 14: return launch_hmc_dmma_w<7, 24>(h, o, n_iter);
+        case 16: return launch_hmc_dmma_w<8, 24>(h, o, n_iter);
+        case 9: return launch_hmc_dmma_w<4, 26>(h, o, n_iter);
+        case 15: return launch_hmc_dmma_w<7, 26>(h, o, n_iter);
+        case 17: return launch_hmc_dmma_w<8, 26>(h, o, n_iter);
         }
+    } else if (M.epilogue) {                // likelihood pipeline: operand streamed from L2
         switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
         case 8: return launch_hmc_dmma_w<4, 8>(h, o, n_iter);
         case 14: return launch_hmc_dmma_w<7, 8>(h, o, n_iter);
@@ -860,22 +844,21 @@ int bfb_launch_hmc_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
         case 15: return launch_hmc_dmma_w<7, 10>(h, o, n_iter);
         case 17: return launch_hmc_dmma_w<8, 10>(h, o, n_iter);
         }
-        return 1;
-    }
-    if (M.frag_nr == 0 || (M.has_c3 && (M.c3_kt == 0 || !M.has_c2))) return 1;
-    if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "dmma")) return 1; }
-    const int mv = (M.has_c2 ? 1 : 0) | (M.frag_ext ? 2 : 0) | (M.has_c3 ? 4 : 0);
+    } else {
+        const int mv = (M.has_c2 ? 1 : 0) | (M.frag_ext ? 2 : 0) | (M.has_c3 ? 4 : 0);
 #ifdef BFB_NO_HEADLINE_SPLIT     // experiment: the headline instantiation inside the big module
-    if (M.frag_nr == 7 && mv == 1) return launch_hmc_dmma_w<7, 1>(h, o, n_iter);
+        if (M.frag_nr == 7 && mv == 1) return launch_hmc_dmma_w<7, 1>(h, o, n_iter);
 #else
-    if (M.frag_nr == 7 && mv == 1) return bfb_launch_hmc_dmma_headline(h, o, n_iter);
+        if (M.frag_nr == 7 && mv == 1) return bfb_launch_hmc_dmma_headline(h, o, n_iter);
 #endif
 #define BFB_CASE(NR_, MV_) if (M.frag_nr == NR_ && mv == MV_) return launch_hmc_dmma_w<NR_, MV_>(h, o, n_iter);
-    BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 2) BFB_CASE(7, 3)
-    BFB_CASE(8, 0) BFB_CASE(8, 1) BFB_CASE(8, 2) BFB_CASE(8, 3)
-    BFB_CASE(4, 5) BFB_CASE(4, 7) BFB_CASE(7, 5) BFB_CASE(7, 7)          // with cubic-3 configs (n <= 28)
+        BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 2) BFB_CASE(7, 3)
+        BFB_CASE(8, 0) BFB_CASE(8, 1) BFB_CASE(8, 2) BFB_CASE(8, 3)
+        BFB_CASE(4, 5) BFB_CASE(4, 7) BFB_CASE(7, 5) BFB_CASE(7, 7)          // with cubic-3 configs (n <= 28)
 #undef BFB_CASE
-    return 1;
+    }
+    bfb_set_error("bfb_launch_hmc_dmma: no kernel instantiation for this model");
+    return BFB_ERR_ARG;
 }
 #endif
 
@@ -900,23 +883,11 @@ static int launch_dmma(bfb_context *h, const bfb_run_out &o, int n_iter, int cpg
     const size_t smem = fixed + sizeof(double) * W * warp_smem_doubles(NR, LS);
     BFB_REQUIRE(smem <= 227 * 1024, BFB_ERR_ARG, "sampler needs %zu bytes of shared memory per block (> 227 KB)", smem);
     BFB_CUDA(cudaFuncSetAttribute(nuts_dmma_kernel<NR, MV, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const size_t deep = (size_t)(L - 1 > LS ? L - 1 - LS : 0) * 3 * SLOT;
-    const size_t prop = (size_t)BFB_NSLOT * 2 * SLOT;
-    if ((deep + prop) * (size_t)n_groups > h->gstack_len) {
-        if (h->gstack) cudaFree(h->gstack);
-        h->gstack = nullptr; h->gstack_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->gstack, sizeof(double) * (deep + prop) * (size_t)n_groups));
-        h->gstack_len = (deep + prop) * (size_t)n_groups;
-    }
+    double *gprop;
+    int rc;
+    if ((rc = gstack_reserve(h, n_groups, L, LS, SLOT, BFB_NSLOT, &gprop))) return rc;
     RunOutDevF od;
     od.o = o; od.n_iter = n_iter;
-    // iteration chunks = work units per group.  A group is bound to ONE warp at a time, but after every chunk it goes back to the queue
-    // and the next free warp takes it: groups migrate between SMs that host 4 busy warps and SMs that host 3 (512 groups on 592 warp
-    // slots), which evens out the finish times.  Measured at 4096 chains x 1500 iterations: 1 / 2 / 6 / 12 / 24 / 48 chunks =
-    // 161 / 154 / 141 / 134.7 / 135.2 / 138.5 ms
-    int chunk_iters = (n_iter + 11) / 12;
-    if (chunk_iters < 16) chunk_iters = n_iter < 16 ? n_iter : 16;
-    if (const char *e = getenv("BFB200_CHUNK_ITERS")) { int v = atoi(e); if (v >= 1) chunk_iters = v; }
     // progress reports for host outputs: chunks of rep_iters iterations counted per CHAIN at its iteration boundary (the work units keep
     // their length: a unit end synchronises the 8 chains of a group, which costs ~3 % of the kernel at 48 units per group)
     const bool report = h->progress_arm > 0;
@@ -926,19 +897,19 @@ static int launch_dmma(bfb_context *h, const bfb_run_out &o, int n_iter, int cpg
         if (rep_iters < 4) rep_iters = n_iter < 4 ? n_iter : 4;
         n_rep = (n_iter + rep_iters - 1) / rep_iters;
     }
-    const int n_chunks = (n_iter + chunk_iters - 1) / chunk_iters;
-    const int64_t n_units64 = (int64_t)n_groups * n_chunks;
-    BFB_REQUIRE(n_units64 < (1ll << 31), BFB_ERR_ARG, "too many work units");
+    // one block per SM whenever there are at least as many groups as SMs: with 512 groups (4096 chains) every SM then runs 3 or
+    // 4 warps instead of 128 SMs running 4 and 20 none
+    int blocks = h->sm_count;
+    if ((int64_t)blocks > n_groups) blocks = n_groups;
+    // iteration chunks = work units per group.  A group is bound to ONE warp at a time, but after every chunk it goes back to the queue
+    // and the next free warp takes it: groups migrate between SMs that host 4 busy warps and SMs that host 3 (512 groups on 592 warp
+    // slots), which evens out the finish times.  Measured at 4096 chains x 1500 iterations: 1 / 2 / 6 / 12 / 24 / 48 chunks =
+    // 161 / 154 / 141 / 134.7 / 135.2 / 138.5 ms
     // work queue, then the progress block (see the iteration boundary of the kernel): 4 + n_rep ints
-    const size_t qlen = 2 + (size_t)n_groups + (size_t)n_units64 + 4 + (size_t)n_rep;
-    if (qlen > h->queue_len) {
-        if (h->queue) cudaFree(h->queue);
-        h->queue = nullptr; h->queue_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->queue, sizeof(int) * qlen));
-        h->queue_len = qlen;
-    }
+    int chunk_iters, n_units;
+    if ((rc = queue_setup(h, n_groups, n_iter, 12, blocks * W, 4 + (size_t)n_rep, chunk_iters, n_units))) return rc;
     {
-        int *pg = h->queue + 2 + (size_t)n_groups + (size_t)n_units64;
+        int *pg = h->queue + 2 + (size_t)n_groups + (size_t)n_units;
         BFB_CUDA(cudaMemsetAsync(pg, 0, sizeof(int) * (4 + (size_t)n_rep), h->stream));
         if (report) {
             const unsigned long long fa = (unsigned long long)h->progress_host_dev;
@@ -947,15 +918,8 @@ static int launch_dmma(bfb_context *h, const bfb_run_out &o, int n_iter, int cpg
             h->progress_chunk_iters = rep_iters; h->progress_n_chunks = n_rep;
         }
     }
-    // one block per SM whenever there are at least as many groups as SMs: with 512 groups (4096 chains) every SM then runs 3 or
-    // 4 warps instead of 128 SMs running 4 and 20 none
-    int blocks = h->sm_count;
-    if ((int64_t)blocks > n_groups) blocks = n_groups;
-    queue_init_kernel<<<(unsigned)((n_units64 + 255) / 256), 256, 0, h->stream>>>(h->queue, n_groups, (int)n_units64, blocks * W);
-    h->launches++;
-    nuts_dmma_kernel<NR, MV, W><<<blocks, 32 * W, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, h->gstack,
-                                                                    h->gstack + deep * (size_t)n_groups, (int)h->iters_done,
-                                                                    chunk_iters, n_groups, (int)n_units64, h->queue, cpg);
+    nuts_dmma_kernel<NR, MV, W><<<blocks, 32 * W, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, h->gstack, gprop,
+                                                                    (int)h->iters_done, chunk_iters, n_groups, n_units, h->queue, cpg);
     h->launches++;
     BFB_CUDA(cudaGetLastError());
     return BFB_OK;
@@ -979,24 +943,21 @@ static int launch_dmma_w(bfb_context *h, const bfb_run_out &o, int n_iter)
 #ifdef BFB_DMMA_PART_HEADLINE
 int bfb_launch_nuts_dmma_headline(bfb_context *h, const bfb_run_out &o, int n_iter) { return launch_dmma_w<7, 1>(h, o, n_iter); }
 #else
-// returns 1 if this path does not apply (caller tries the next kernel), 0 on launch, <0 on error
+// launches the NUTS kernel of the model (select_family, bfb_sampler.cu, chose this family): 0 on launch, 1 when its shared memory
+// does not fit, < 0 on error
 int bfb_launch_nuts_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     const DevModel &M = h->dm;
-    if (M.epilogue) {                       // likelihood pipeline (model variant bit 3): operand streamed from L2
-        if (!M.lik_tab || h->scfg.max_treedepth > 10) return 1;
-        if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "dmma")) return 1; }
-        if (M.lik_ftab) {                 // feature form: two chained GEMMs per 8 outputs (model variant bit 4)
-            switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
-            case 8: return launch_dmma_w<4, 24>(h, o, n_iter);
-            case 14: return launch_dmma_w<7, 24>(h, o, n_iter);
-            case 16: return launch_dmma_w<8, 24>(h, o, n_iter);
-            case 9: return launch_dmma_w<4, 26>(h, o, n_iter);
-            case 15: return launch_dmma_w<7, 26>(h, o, n_iter);
-            case 17: return launch_dmma_w<8, 26>(h, o, n_iter);
-            }
-            return 1;
+    if (M.epilogue && M.lik_ftab) {         // likelihood pipeline (model variant bit 3), feature form: two chained GEMMs per 8 outputs (bit 4)
+        switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
+        case 8: return launch_dmma_w<4, 24>(h, o, n_iter);
+        case 14: return launch_dmma_w<7, 24>(h, o, n_iter);
+        case 16: return launch_dmma_w<8, 24>(h, o, n_iter);
+        case 9: return launch_dmma_w<4, 26>(h, o, n_iter);
+        case 15: return launch_dmma_w<7, 26>(h, o, n_iter);
+        case 17: return launch_dmma_w<8, 26>(h, o, n_iter);
         }
+    } else if (M.epilogue) {                // likelihood pipeline: operand streamed from L2
         switch (M.lik_nr * 2 + (M.lik_ext ? 1 : 0)) {
         case 8: return launch_dmma_w<4, 8>(h, o, n_iter);
         case 14: return launch_dmma_w<7, 8>(h, o, n_iter);
@@ -1005,23 +966,21 @@ int bfb_launch_nuts_dmma(bfb_context *h, const bfb_run_out &o, int n_iter)
         case 15: return launch_dmma_w<7, 10>(h, o, n_iter);
         case 17: return launch_dmma_w<8, 10>(h, o, n_iter);
         }
-        return 1;
-    }
-    if (M.frag_nr == 0 || (M.has_c3 && (M.c3_kt == 0 || !M.has_c2))) return 1;
-    if (h->scfg.max_treedepth > 10) return 1;
-    if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "dmma")) return 1; }
-    const int mv = (M.has_c2 ? 1 : 0) | (M.frag_ext ? 2 : 0) | (M.has_c3 ? 4 : 0);
+    } else {
+        const int mv = (M.has_c2 ? 1 : 0) | (M.frag_ext ? 2 : 0) | (M.has_c3 ? 4 : 0);
 #ifdef BFB_NO_HEADLINE_SPLIT
-    if (M.frag_nr == 7 && mv == 1) return launch_dmma_w<7, 1>(h, o, n_iter);
+        if (M.frag_nr == 7 && mv == 1) return launch_dmma_w<7, 1>(h, o, n_iter);
 #else
-    if (M.frag_nr == 7 && mv == 1) return bfb_launch_nuts_dmma_headline(h, o, n_iter);
+        if (M.frag_nr == 7 && mv == 1) return bfb_launch_nuts_dmma_headline(h, o, n_iter);
 #endif
 #define BFB_CASE(NR_, MV_) if (M.frag_nr == NR_ && mv == MV_) return launch_dmma_w<NR_, MV_>(h, o, n_iter);
-    BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 2) BFB_CASE(7, 3)
-    BFB_CASE(8, 0) BFB_CASE(8, 1) BFB_CASE(8, 2) BFB_CASE(8, 3)
-    BFB_CASE(4, 5) BFB_CASE(4, 7) BFB_CASE(7, 5) BFB_CASE(7, 7)          // with cubic-3 configs (n <= 28)
+        BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 2) BFB_CASE(7, 3)
+        BFB_CASE(8, 0) BFB_CASE(8, 1) BFB_CASE(8, 2) BFB_CASE(8, 3)
+        BFB_CASE(4, 5) BFB_CASE(4, 7) BFB_CASE(7, 5) BFB_CASE(7, 7)          // with cubic-3 configs (n <= 28)
 #undef BFB_CASE
-    return 1;
+    }
+    bfb_set_error("bfb_launch_nuts_dmma: no kernel instantiation for this model");
+    return BFB_ERR_ARG;
 }
 #endif
 

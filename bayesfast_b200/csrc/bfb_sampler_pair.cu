@@ -771,63 +771,38 @@ static int launch_pair(bfb_context *h, const bfb_run_out &o, int n_iter)
     const int n_groups = (int)((C + 7) / 8);
     const size_t fixed = sizeof(double) * (SH::frag_doubles(NP) + SH::MSM_DOUBLES + (SH::C3 ? dmma_c3_doubles(NR, h->dm.c3_kt, NP) : 0));
     const size_t cap = 227 * 1024;
-    if (fixed + sizeof(double) * NP * pair_smem_doubles(NR, 1) > cap) return 1;          // does not fit: the one-warp kernel
+    if (fixed + sizeof(double) * NP * pair_smem_doubles(NR, 1) > cap) return 1;          // does not fit
     int LS = L - 1 > 1 ? L - 1 : 1;
     while (LS > 1 && fixed + sizeof(double) * NP * pair_smem_doubles(NR, LS) > cap) --LS;
     if (const char *e = getenv("BFB200_STACK_LEVELS_SMEM")) { int v = atoi(e); if (v >= 1 && v < LS) LS = v; }
     const size_t smem = fixed + sizeof(double) * NP * pair_smem_doubles(NR, LS);
     BFB_CUDA(cudaFuncSetAttribute(nuts_pair_kernel<NR, MV, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const size_t deep = (size_t)(L - 1 > LS ? L - 1 - LS : 0) * 3 * SLOT;
-    const size_t prop = (size_t)BFB_PAIR_NSLOT * 2 * SLOT;
-    if ((deep + prop) * (size_t)n_groups > h->gstack_len) {
-        if (h->gstack) cudaFree(h->gstack);
-        h->gstack = nullptr; h->gstack_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->gstack, sizeof(double) * (deep + prop) * (size_t)n_groups));
-        h->gstack_len = (deep + prop) * (size_t)n_groups;
-    }
+    double *gprop;
+    int rc;
+    if ((rc = gstack_reserve(h, n_groups, L, LS, SLOT, BFB_PAIR_NSLOT, &gprop))) return rc;
     RunOutDevF od;
     od.o = o; od.n_iter = n_iter;
-    int chunk_iters = (n_iter + 5) / 6;
-    if (chunk_iters < 16) chunk_iters = n_iter < 16 ? n_iter : 16;
-    if (const char *e = getenv("BFB200_CHUNK_ITERS")) { int v = atoi(e); if (v >= 1) chunk_iters = v; }
-    const int n_chunks = (n_iter + chunk_iters - 1) / chunk_iters;
-    const int64_t n_units64 = (int64_t)n_groups * n_chunks;
-    BFB_REQUIRE(n_units64 < (1ll << 31), BFB_ERR_ARG, "too many work units");
-    const size_t qlen = 2 + (size_t)n_groups + (size_t)n_units64;
-    if (qlen > h->queue_len) {
-        if (h->queue) cudaFree(h->queue);
-        h->queue = nullptr; h->queue_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->queue, sizeof(int) * qlen));
-        h->queue_len = qlen;
-    }
     int blocks = h->sm_count;
     if ((int64_t)blocks > n_groups) blocks = n_groups;
-    queue_init_kernel<<<(unsigned)((n_units64 + 255) / 256), 256, 0, h->stream>>>(h->queue, n_groups, (int)n_units64, blocks * NP);
-    h->launches++;
-    nuts_pair_kernel<NR, MV, NP><<<blocks, 64 * NP, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, h->gstack,
-                                                                       h->gstack + deep * (size_t)n_groups, (int)h->iters_done,
-                                                                       chunk_iters, n_groups, (int)n_units64, h->queue);
+    int chunk_iters, n_units;
+    if ((rc = queue_setup(h, n_groups, n_iter, 6, blocks * NP, 0, chunk_iters, n_units))) return rc;
+    nuts_pair_kernel<NR, MV, NP><<<blocks, 64 * NP, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, h->gstack, gprop,
+                                                                       (int)h->iters_done, chunk_iters, n_groups, n_units, h->queue);
     h->launches++;
     BFB_CUDA(cudaGetLastError());
     return BFB_OK;
 }
 
-// returns 1 if this path does not apply (caller tries the next kernel), 0 on launch, <0 on error
+// launches the pair kernel of the model (select_family, bfb_sampler.cu, chose this family): 0 on launch, 1 when its shared memory
+// does not fit, < 0 on error
 int bfb_launch_nuts_pair(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     const DevModel &M = h->dm;
-    if (M.epilogue) return 1;
-    if (M.frag_nr == 0 || M.has_c3) return 1;
-    if (h->scfg.max_treedepth > 10) return 1;
-    const char *e = getenv("BFB200_SAMPLER");
-    if (!e || strcmp(e, "pair")) return 1;
     const int mv = (M.has_c2 ? 1 : 0) | (M.frag_ext ? 2 : 0);
 #define BFB_CASE(NR_, MV_) if (M.frag_nr == NR_ && mv == MV_) return launch_pair<NR_, MV_>(h, o, n_iter);
-    BFB_CASE(7, 1)
-#ifndef BFB_PAIR_HEADLINE_ONLY
-    BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 2) BFB_CASE(7, 3)
+    BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(4, 2) BFB_CASE(4, 3) BFB_CASE(7, 0) BFB_CASE(7, 1) BFB_CASE(7, 2) BFB_CASE(7, 3)
     BFB_CASE(8, 0) BFB_CASE(8, 1) BFB_CASE(8, 2) BFB_CASE(8, 3)
-#endif
 #undef BFB_CASE
-    return 1;
+    bfb_set_error("bfb_launch_nuts_pair: no kernel instantiation for this model");
+    return BFB_ERR_ARG;
 }

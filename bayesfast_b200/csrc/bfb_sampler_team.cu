@@ -1,5 +1,6 @@
 // bfb_sampler_team.cu -- NUTS / HMC with EIGHT chains per TEAM of four warps (bfb_team.cuh): the tensor-core sampler for
-// linear + quadratic (+ cubic-2) surrogates with or without radial bound, input_size <= 32.
+// linear + quadratic (+ cubic-2, + cubic-3 above 32 dimensions) surrogates with or without radial bound, HMC for input_size
+// <= 64, NUTS for 32 < input_size <= 64.
 //
 // Reference restated here: samplers/hmc_utils/base_hmc.py:62-85, samplers/nuts.py:27-217, samplers/hmc.py:16-49,
 // hmc_utils/integration.py:28-95, hmc_utils/metrics.py:73-91,186-211,333-371, hmc_utils/step_size.py:10-51.
@@ -22,17 +23,6 @@ static __device__ __noinline__ void team_dual_average(double cnt, double hbar0, 
     const double mk = pow(cnt, -kk);
     log_bar_new = mk * log_step + (1. - mk) * log_bar;
     e_step = exp(log_step); e_bar = exp(log_bar_new);
-}
-
-// Work queue (same layout as queue_init_kernel, bfb_nuts_common.cuh), but the first `head0` units are pre-assigned: team
-// slot s = blockIdx.x + gridDim.x * team takes unit s without an atomic, so that the teams of ALL blocks get work when there
-// are fewer groups than team slots (4096 chains = 512 groups on 148 x 4 = 592 slots).
-static __global__ void team_queue_init_kernel(int *queue, int n_groups, int n_units, int head0)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) { queue[0] = head0; queue[1] = n_groups; }
-    if (i < n_groups) queue[2 + i] = 0;
-    if (i < n_units) queue[2 + n_groups + i] = (i < n_groups) ? i : -1;
 }
 
 // shared memory of a team of the HMC kernel: exchange buffers (x | x - mu | x^2) | reduction buffers | control words
@@ -265,27 +255,6 @@ __global__ void __launch_bounds__(128 * G, 1) hmc_team_kernel(DevModel M, bfb_sa
     }   // unit loop
 }
 
-static int team_queue_setup(bfb_context *h, int n_groups, int n_iter, int slots, int &chunk_iters, int &n_units)
-{
-    chunk_iters = (n_iter + 5) / 6;
-    if (chunk_iters < 16) chunk_iters = n_iter < 16 ? n_iter : 16;
-    if (const char *e = getenv("BFB200_CHUNK_ITERS")) { int v = atoi(e); if (v >= 1) chunk_iters = v; }
-    const int n_chunks = (n_iter + chunk_iters - 1) / chunk_iters;
-    const int64_t n_units64 = (int64_t)n_groups * n_chunks;
-    BFB_REQUIRE(n_units64 < (1ll << 31), BFB_ERR_ARG, "too many work units");
-    n_units = (int)n_units64;
-    const size_t qlen = 2 + (size_t)n_groups + (size_t)n_units64;
-    if (qlen > h->queue_len) {
-        if (h->queue) cudaFree(h->queue);
-        h->queue = nullptr; h->queue_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->queue, sizeof(int) * qlen));
-        h->queue_len = qlen;
-    }
-    team_queue_init_kernel<<<(unsigned)((n_units64 + 255) / 256), 256, 0, h->stream>>>(h->queue, n_groups, n_units, slots);
-    h->launches++;
-    return BFB_OK;
-}
-
 template <int NR, int MV, int G>
 static int launch_hmc_team(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
@@ -300,7 +269,7 @@ static int launch_hmc_team(bfb_context *h, const bfb_run_out &o, int n_iter)
     int blocks = h->sm_count;
     if ((int64_t)blocks > n_groups) blocks = n_groups;
     int chunk_iters, n_units, rc;
-    if ((rc = team_queue_setup(h, n_groups, n_iter, blocks * G, chunk_iters, n_units))) return rc;
+    if ((rc = queue_setup(h, n_groups, n_iter, 6, blocks * G, 0, chunk_iters, n_units))) return rc;
     hmc_team_kernel<NR, MV, G><<<blocks, 128 * G, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, (int)h->iters_done, chunk_iters,
                                                                     n_groups, n_units, h->queue);
     h->launches++;
@@ -321,28 +290,21 @@ static int launch_hmc_team_g(bfb_context *h, const bfb_run_out &o, int n_iter)
     return launch_hmc_team<NR, MV, 4>(h, o, n_iter);
 }
 
-// returns 1 if this path does not apply (caller tries the next kernel), 0 on launch, <0 on error
+// launches the HMC kernel of the model (select_family, bfb_sampler.cu, chose this family): 0 on launch, 1 when its shared memory
+// does not fit, < 0 on error
 int bfb_launch_hmc_team(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     const DevModel &M = h->dm;
-    if (M.epilogue || !M.tfrag || M.team_nr == 0 || M.frag_ext) return 1;
-    if (M.has_c3 && !(M.team_nr == 16 && M.tfrag3 && M.has_c2)) return 1;
-    if (M.team_nr == 16) {
-        // 32 < n <= 64: the only tensor-core path (the one-warp kernels hold at most 8 dimensions per lane); one team per SM (the
-        // operand table alone is 128 KB), more groups than SMs queue
-        if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "team")) return 1; }
+    if (M.team_nr == 16) {            // 32 < n <= 64: one team per SM (the operand table alone is 128 KB), more groups than SMs queue
         if (M.has_c3) return launch_hmc_team<16, 5, 1>(h, o, n_iter);
         return M.has_c2 ? launch_hmc_team<16, 1, 1>(h, o, n_iter) : launch_hmc_team<16, 0, 1>(h, o, n_iter);
     }
-    // default for up to four groups per SM (4736 chains on a B200): 4096 chains 2.20e9 leapfrogs/s here against 2.06e9 with one
-    // warp per group; above that the one-warp kernel has enough warps and fewer instructions (16384 chains: 2.5e9 against 3.2e9)
-    if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "team")) return 1; }
-    else if ((h->cs.C + 7) / 8 > (int64_t)h->sm_count * 4) return 1;
     const int mv = M.has_c2 ? 1 : 0;
 #define BFB_CASE(NR_, MV_) if (M.team_nr == NR_ && mv == MV_) return launch_hmc_team_g<NR_, MV_>(h, o, n_iter);
     BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(7, 0) BFB_CASE(7, 1) BFB_CASE(8, 0) BFB_CASE(8, 1)
 #undef BFB_CASE
-    return 1;
+    bfb_set_error("bfb_launch_hmc_team: no kernel instantiation for this model");
+    return BFB_ERR_ARG;
 }
 
 // ----------------------------------------------------------------------------------------------------------------------
@@ -376,11 +338,11 @@ int bfb_launch_hmc_team(bfb_context *h, const bfb_run_out &o, int n_iter)
 // doubles of shared memory per team: 14 fixed vector slots + 3 per stack level 1..LS | reduction | per-level scalars | flags
 __host__ __device__ inline int team_nuts_doubles(int slot, int LS) { return (14 + 3 * LS) * slot + 256 + 400 + 96; }
 
-template <int NR, int MV, int G>
-__global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_sampler_cfg cfg, ChainState st, RunOutDevF out,
-                                                               int L, int LS, int tstride, double *__restrict__ gstack,
-                                                               double *__restrict__ gprop, int base_iter, int chunk_iters,
-                                                               int n_groups, int n_units, int *__restrict__ queue)
+template <int NR, int MV>
+__global__ void __launch_bounds__(128, 1) nuts_team_kernel(DevModel M, bfb_sampler_cfg cfg, ChainState st, RunOutDevF out,
+                                                           int L, int LS, double *__restrict__ gstack, double *__restrict__ gprop,
+                                                           int base_iter, int chunk_iters, int n_groups, int n_units,
+                                                           int *__restrict__ queue)
 {
     using TS = TeamShape<NR, MV>;
     constexpr int NRW = TS::NRW, SLOT = TS::SLOT;
@@ -389,9 +351,9 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
     for (int i = threadIdx.x; i < TS::TAB_DOUBLES; i += blockDim.x) tab[i] = M.tfrag[i];
     for (int i = threadIdx.x; i < TS::MSM_HALF && i < M.np; i += blockDim.x) { msm[i] = M.use_bound ? M.mu[i] : 0.; msm[TS::MSM_HALF + i] = M.lin[i]; }
     __syncthreads();
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, team = wib >> 2, w = wib & 3, gi = lane >> 2, lg = lane & 3;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, gi = lane >> 2, lg = lane & 3;
     const int cc = 2 * w + (lane >> 4), cl = lane & 15;         // control chain of this lane, lane index within its half warp
-    double *tsm = smem + TS::TAB_DOUBLES + TS::MSM + team * tstride;
+    double *tsm = smem + TS::TAB_DOUBLES + TS::MSM;
     double *xb = tsm, *sRL = tsm + SLOT, *sRS = tsm + 2 * SLOT, *sPBUF = tsm + 3 * SLOT;
     double *sTLQ = tsm + 4 * SLOT, *sTLP = tsm + 5 * SLOT, *sTLG = tsm + 6 * SLOT;
     double *sTRQ = tsm + 7 * SLOT, *sTRP = tsm + 8 * SLOT, *sTRG = tsm + 9 * SLOT;
@@ -403,7 +365,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
     volatile int *ci = reinterpret_cast<volatile int *>(flg);     // [0, 8) command words | [8, 20) level flags | 20 extend flags | 24 unit
     // [0,8) step | [8,16) logp | [16,24) draw counter | [24,32) kinetic energy | [32,40) first direction draw | [40,48) leaf logp | [48,56) leaf energy
     volatile double *cdv = flg + 16;
-    const int bar_id = 1 + team;
+    const int bar_id = 1;
     const double *tab_w = tab + (size_t)w * NR * TS::NTW * 32;
     const double *mu_t = msm;
     const bool leader = (w == 0 && lane == 0), chief = (cl == 0);
@@ -413,7 +375,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
     volatile int *ring = queue + 2 + n_groups;
     int rbuf = 0;
     bool first = true;
-    const int slot_id = blockIdx.x + gridDim.x * team;
+    const int slot_id = blockIdx.x;
 #ifdef BFB_TEAM_TIMING     // per-phase cycle counters of warp 0 (printed with BFB200_DEBUG=1)
 #define TTICK(k_) { const long long now_ = clock64(); tacc[k_] += now_ - tlast; tlast = now_; }
 #else
@@ -565,7 +527,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
                 // lane n draws the uniform that follows the normals: the direction of the first doubling (nuts.py:210)
                 {
                     unsigned mask = __ballot_sync(BFB_FULL, startp && !done) & 0x11111111u;
-                    int idx = team;
+                    int idx = 0;
 #pragma unroll 1
                     while (mask) {
                         const int src = __ffs(mask) - 1;
@@ -706,7 +668,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
         // ================= tasks: U-turn dot products of all merges of this leaf and of Tree.extend =================
 #pragma unroll 1
         for (int l = 0; l < kmax; ++l) {
-            if (((l + team) & 3) != w) continue;
+            if ((l & 3) != w) continue;
             double v0 = 0., v1 = 0., v2 = 1., v3 = 1., v4 = 1., v5 = 1.;
             if (l == 0) {
 #pragma unroll
@@ -756,7 +718,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
             const unsigned bal = __ballot_sync(BFB_FULL, turning);
             if (lane == 0) ci[8 + l] = (int)bal;
         }
-        if (((3 + team) & 3) == w && __any_sync(BFB_FULL, last)) {
+        if (w == 3 && __any_sync(BFB_FULL, last)) {
             // Tree.extend, nuts.py:86-101 (self.p_sum is updated in place BEFORE p_sum1 / p_sum2 are formed)
             const bool right = step > 0.;
             double v0 = 0., v1 = 0., v2 = 0., v3 = 0., v4 = 0., v5 = 0.;
@@ -950,7 +912,7 @@ __global__ void __launch_bounds__(128 * G, 1) nuts_team_kernel(DevModel M, bfb_s
 #undef OST
 }
 
-template <int NR, int MV, int G>
+template <int NR, int MV>
 static int launch_nuts_team(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     using TS = TeamShape<NR, MV>;
@@ -958,72 +920,36 @@ static int launch_nuts_team(bfb_context *h, const bfb_run_out &o, int n_iter)
     const int L = h->scfg.max_treedepth;
     const int64_t C = h->cs.C;
     const int n_groups = (int)((C + 7) / 8);
-    // stack levels 1..LS in shared memory, deeper (rarely touched) levels in an L2-resident buffer
+    // one team per SM (the operand table alone is 128 KB), more groups than SMs queue; stack levels 1..LS in shared memory,
+    // deeper (rarely touched) levels in an L2-resident buffer
     const size_t fixed = sizeof(double) * (TS::TAB_DOUBLES + TS::MSM);
     int LS = L - 1;
-    while (LS > 0 && fixed + sizeof(double) * G * team_nuts_doubles(SLOT, LS) > (size_t)(227 * 1024)) --LS;
+    while (LS > 0 && fixed + sizeof(double) * team_nuts_doubles(SLOT, LS) > (size_t)(227 * 1024)) --LS;
     if (const char *e = getenv("BFB200_STACK_LEVELS_SMEM")) { int v = atoi(e); if (v >= 0 && v < LS) LS = v; }
-    const size_t smem = fixed + sizeof(double) * G * team_nuts_doubles(SLOT, LS);
+    const size_t smem = fixed + sizeof(double) * team_nuts_doubles(SLOT, LS);
     if (smem > (size_t)(227 * 1024)) return 1;
-    BFB_CUDA(cudaFuncSetAttribute(nuts_team_kernel<NR, MV, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const size_t deep = (size_t)(L - 1 > LS ? L - 1 - LS : 0) * 3 * SLOT;
-    const size_t prop = (size_t)BFB_NSLOT * 2 * SLOT;
-    if ((deep + prop) * (size_t)n_groups > h->gstack_len) {
-        if (h->gstack) cudaFree(h->gstack);
-        h->gstack = nullptr; h->gstack_len = 0;
-        BFB_CUDA(cudaMalloc((void **)&h->gstack, sizeof(double) * (deep + prop) * (size_t)n_groups));
-        h->gstack_len = (deep + prop) * (size_t)n_groups;
-    }
+    BFB_CUDA(cudaFuncSetAttribute(nuts_team_kernel<NR, MV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    double *gprop;
+    int rc;
+    if ((rc = gstack_reserve(h, n_groups, L, LS, SLOT, BFB_NSLOT, &gprop))) return rc;
     RunOutDevF od;
     od.o = o; od.n_iter = n_iter;
     int blocks = h->sm_count;
     if ((int64_t)blocks > n_groups) blocks = n_groups;
-    int chunk_iters, n_units, rc;
-    if ((rc = team_queue_setup(h, n_groups, n_iter, blocks * G, chunk_iters, n_units))) return rc;
-    nuts_team_kernel<NR, MV, G><<<blocks, 128 * G, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, team_nuts_doubles(SLOT, LS), h->gstack,
-                                                                     h->gstack + deep * (size_t)n_groups, (int)h->iters_done,
-                                                                     chunk_iters, n_groups, n_units, h->queue);
+    int chunk_iters, n_units;
+    if ((rc = queue_setup(h, n_groups, n_iter, 6, blocks, 0, chunk_iters, n_units))) return rc;
+    nuts_team_kernel<NR, MV><<<blocks, 128, smem, h->stream>>>(h->dm, h->scfg, h->cs, od, L, LS, h->gstack, gprop, (int)h->iters_done,
+                                                               chunk_iters, n_groups, n_units, h->queue);
     h->launches++;
     BFB_CUDA(cudaGetLastError());
     return BFB_OK;
 }
 
-template <int NR, int MV>
-static int launch_nuts_team_g(bfb_context *h, const bfb_run_out &o, int n_iter)
-{
-    // teams per SM: 3 (168 registers, no spills; 4 teams cap the kernel at 128 registers and run every phase ~1.5x slower).
-    // Fewer team slots than groups is fine: the groups' iteration chunks are dealt to the slots by the work queue.
-    int G = 3;
-    if (const char *e = getenv("BFB200_TEAMS_PER_SM")) { int v = atoi(e); if (v >= 1 && v <= 5) G = v; }
-    switch (G) {
-    case 1: return launch_nuts_team<NR, MV, 1>(h, o, n_iter);
-    case 2: return launch_nuts_team<NR, MV, 2>(h, o, n_iter);
-    case 4: return launch_nuts_team<NR, MV, 4>(h, o, n_iter);
-    case 5: return launch_nuts_team<NR, MV, 5>(h, o, n_iter);
-    }
-    return launch_nuts_team<NR, MV, 3>(h, o, n_iter);
-}
-
-// returns 1 if this path does not apply (caller tries the next kernel), 0 on launch, <0 on error
+// launches the NUTS kernel of the model (select_family, bfb_sampler.cu, chose this family: 32 < n <= 64): 0 on launch, 1 when
+// its shared memory does not fit, < 0 on error
 int bfb_launch_nuts_team(bfb_context *h, const bfb_run_out &o, int n_iter)
 {
     const DevModel &M = h->dm;
-    if (M.epilogue || !M.tfrag || M.team_nr == 0 || M.frag_ext) return 1;
-    if (M.has_c3 && !(M.team_nr == 16 && M.tfrag3 && M.has_c2)) return 1;
-    if (h->scfg.max_treedepth > 10 || h->scfg.max_treedepth < 1) return 1;
-    if (M.team_nr == 16) {
-        // 32 < n <= 64 (BASELINE configs[3]: 64-D cubic-3): the only tensor-core path, default; one team per SM
-        if (const char *e = getenv("BFB200_SAMPLER")) { if (strcmp(e, "team")) return 1; }
-        if (M.has_c3) return launch_nuts_team<16, 5, 1>(h, o, n_iter);
-        return M.has_c2 ? launch_nuts_team<16, 1, 1>(h, o, n_iter) : launch_nuts_team<16, 0, 1>(h, o, n_iter);
-    }
-    // Measured (d = 26 cubic-2, B200, profiles/r02_a_team_*): one group alone on an SM makes a leaf in 6.8 k cycles here against
-    // 10 k on the one-warp-per-group kernel, but three resident teams slow each other to 10.6 k (4096 chains: 5.2e8 against
-    // 7.1e8 leapfrogs/s), so the one-warp kernel stays the default and this one is selected with BFB200_SAMPLER=team.
-    { const char *e = getenv("BFB200_SAMPLER"); if (!e || strcmp(e, "team")) return 1; }
-    const int mv = M.has_c2 ? 1 : 0;
-#define BFB_CASE(NR_, MV_) if (M.team_nr == NR_ && mv == MV_) return launch_nuts_team_g<NR_, MV_>(h, o, n_iter);
-    BFB_CASE(4, 0) BFB_CASE(4, 1) BFB_CASE(7, 0) BFB_CASE(7, 1) BFB_CASE(8, 0) BFB_CASE(8, 1)
-#undef BFB_CASE
-    return 1;
+    if (M.has_c3) return launch_nuts_team<16, 5>(h, o, n_iter);
+    return M.has_c2 ? launch_nuts_team<16, 1>(h, o, n_iter) : launch_nuts_team<16, 0>(h, o, n_iter);
 }

@@ -212,8 +212,9 @@ int bfb_tsampler_run(bfb_handle h, int sampler, int32_t n_iter, const bfb_run_ou
                      int64_t *total_tree_size);
 /* which kernel family ran the last bfb_sampler_run / bfb_tsampler_run of this handle: 0 = warp-per-chain (bfb_sampler.cu,
  * bfb_sampler_tempered.cu), 2 = FP64 tensor core, one warp per 8 chains (bfb_sampler_dmma.cu), 3 = tensor core, four-warp team per
- * 8 chains (bfb_sampler_team.cu), 4 = tensor core, integrator warp + tree warp (bfb_sampler_pair.cu); -1 before the first run.
- * The environment variable BFB200_SAMPLER = dmma | team | pair | generic pins one (tests, profiles). */
+ * 8 chains (bfb_sampler_team.cu; NUTS for 32 < n <= 64 only), 4 = tensor core, integrator warp + tree warp (bfb_sampler_pair.cu,
+ * NUTS only); -1 before the first run.  The environment variable BFB200_SAMPLER = dmma | team | pair | generic pins one (tests,
+ * profiles); bfb_sampler_run fails with BFB_ERR_ARG when the pinned family cannot run the model. */
 int bfb_sampler_last_path(bfb_handle h);
 /* page-locked host memory for the outputs of bfb_sampler_run: with it the device-to-host copies of one chunk of
  * iterations overlap the kernel of the next chunk */

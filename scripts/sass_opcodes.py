@@ -5,7 +5,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CS = os.path.join(ROOT, 'bayesfast_b200', 'csrc')
 KERNELS = [('bfb_sampler_dmma_headline.o', 'nuts_dmma_kernelILi7ELi1ELi4E', 'nuts_dmma_kernel<7,1,4> (headline: d=26 cubic-2 NUTS, 8 chains per warp)'),
            ('bfb_sampler_dmma_headline.o', 'hmc_dmma_kernelILi7ELi1ELi8E', 'hmc_dmma_kernel<7,1,8>'),
-           ('bfb_sampler_team.o', 'nuts_team_kernelILi7ELi1ELi3E', 'nuts_team_kernel<7,1,3> (8 chains per team of four warps)'),
+           ('bfb_sampler_team.o', 'nuts_team_kernelILi16ELi5EE', 'nuts_team_kernel<16,5> (64-D cubic-3, 8 chains per team of four warps)'),
            ('bfb_sampler_team.o', 'hmc_team_kernelILi7ELi1ELi4E', 'hmc_team_kernel<7,1,4>'),
            ('bfb_sampler_pair.o', 'nuts_pair_kernelILi7ELi1ELi4E', 'nuts_pair_kernel<7,1,4> (integrator warp + tree warp per 8-chain group)'),
            ('bfb_sampler_dmma.o', 'nuts_dmma_kernelILi7ELi10ELi4E', 'nuts_dmma_kernel<7,10,4> (DES-shaped likelihood pipeline: bound + rescale + transform + prior)'),

@@ -1,4 +1,4 @@
-"""debug: team NUTS vs oracle float differences per iteration"""
+"""debug: tensor-core NUTS (BFB200_SAMPLER family, default dmma) vs oracle float differences per iteration"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
@@ -9,7 +9,7 @@ from _specs import synthetic_spec, to_device_spec
 from test_gpu_sampler import cfg_from, device_draws
 bf_oracle.build()
 n, order, C, n_iter = 16, 'cubic-2', 70, 40
-fam = sys.argv[1] if len(sys.argv) > 1 else 'team'
+fam = sys.argv[1] if len(sys.argv) > 1 else 'dmma'
 os.environ['BFB200_SAMPLER'] = fam
 h = _cabi.Handle(0)
 spec, cov = synthetic_spec(n, order, seed=70 + n)

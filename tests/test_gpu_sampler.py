@@ -289,7 +289,8 @@ def test_work_queue_chunking_is_invisible(handle, monkeypatch):
             assert np.array_equal(o[k], outs[0][k]), k
 
 
-@pytest.mark.parametrize('n,order,C,n_iter,env', [
+# n, order, chains, iterations, environment of the one-warp (dmma) and pair kernels (n <= 32) ...
+NUTS_CASES = [
     (26, 'cubic-2', 203, 40, {}),                                  # ragged: 203 = 25 groups of 8 + 3 chains
     (26, 'cubic-2', 203, 40, {'BFB200_WARPS_PER_SM': '8'}),        # the 8-warps-per-SM launch used above 4736 chains
     (26, 'cubic-2', 64, 48, {'BFB200_STACK_LEVELS_SMEM': '1', 'BFB200_CHUNK_ITERS': '7'}),   # deep stack levels in L2, odd chunks
@@ -297,14 +298,31 @@ def test_work_queue_chunking_is_invisible(handle, monkeypatch):
     (31, 'cubic-2', 40, 30, {}),
     (5, 'cubic-2', 50, 40, {}),
     (26, 'quadratic', 100, 40, {}),
-    (26, 'cubic-2', 203, 40, {'BFB200_TEAMS_PER_SM': '3', 'BFB200_STACK_LEVELS_SMEM': '0'}),
-    (16, 'quadratic', 33, 40, {'BFB200_TEAMS_PER_SM': '5', 'BFB200_CHUNK_ITERS': '9'}),
-])
-@pytest.mark.parametrize('family', ['team', 'dmma', 'pair'])
+    (26, 'cubic-2', 203, 40, {'BFB200_STACK_LEVELS_SMEM': '0'}),
+    (16, 'quadratic', 33, 40, {'BFB200_CHUNK_ITERS': '9'}),
+]
+# ... and of the team kernel (32 < n <= 64)
+TEAM_NUTS_CASES = [
+    (40, 'cubic-2', 203, 40, {}),
+    (40, 'cubic-2', 64, 48, {'BFB200_STACK_LEVELS_SMEM': '1', 'BFB200_CHUNK_ITERS': '7'}),
+    (48, 'cubic-2', 70, 40, {}),
+    (64, 'cubic-2', 40, 30, {}),
+    (33, 'cubic-2', 50, 40, {}),
+    (40, 'quadratic', 100, 40, {}),
+    (40, 'cubic-2', 203, 40, {'BFB200_STACK_LEVELS_SMEM': '0'}),
+    (56, 'quadratic', 33, 40, {'BFB200_CHUNK_ITERS': '9'}),
+    (40, 'cubic-3', 21, 24, {'BFB200_STACK_LEVELS_SMEM': '2'}),
+]
+
+
+@pytest.mark.parametrize('family,n,order,C,n_iter,env', [
+    pytest.param(f, *c, id='%s-%d-%s-%d-%d-env%d' % (f, c[0], c[1], c[2], c[3], i))
+    for f, cases in (('dmma', NUTS_CASES), ('pair', NUTS_CASES), ('team', TEAM_NUTS_CASES)) for i, c in enumerate(cases)])
 def test_tensor_core_nuts_vs_oracle(handle, oracle, monkeypatch, n, order, C, n_iter, env, family):
-    """bfb_sampler_team.cu (8 chains per team of four warps) / bfb_sampler_dmma.cu (8 chains per warp) / bfb_sampler_pair.cu
-    (integrator warp + tree warp per 8 chains, speculative trajectory), the chains as the rows of FP64 DMMAs: per-chain tree depths / sizes / divergences and draw counts identical to the oracle fed with the device's
-    own draws, and to the generic warp-per-chain kernel"""
+    """bfb_sampler_dmma.cu (8 chains per warp) / bfb_sampler_pair.cu (integrator warp + tree warp per 8 chains, speculative
+    trajectory) / bfb_sampler_team.cu (8 chains per team of four warps, 32 < n <= 64), the chains as the rows of FP64 DMMAs:
+    per-chain tree depths / sizes / divergences and draw counts identical to the oracle fed with the device's own draws, and
+    to the generic warp-per-chain kernel"""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     monkeypatch.setenv('BFB200_SAMPLER', family)
@@ -343,11 +361,11 @@ def test_tensor_core_nuts_vs_oracle(handle, oracle, monkeypatch, n, order, C, n_
         assert np.array_equal(out[k], gen[k]), k
 
 
-@pytest.mark.parametrize('family', ['team', 'dmma', 'pair'])
-def test_tensor_core_nuts_resume_and_reset(handle, monkeypatch, family):
+@pytest.mark.parametrize('family,n,C', [('dmma', 26, 96), ('pair', 26, 96), ('team', 40, 101)],    # 101 chains: a ragged group
+                         ids=['dmma', 'pair', 'team-n40'])
+def test_tensor_core_nuts_resume_and_reset(handle, monkeypatch, family, n, C):
     """chain state survives between launches (bfb_sampler_run called twice == once), and bfb_sampler_reset restarts it"""
     monkeypatch.setenv('BFB200_SAMPLER', family)
-    n, C = 26, 96
     spec, cov = synthetic_spec(n, 'cubic-2', seed=12)
     handle.set_model(to_device_spec(spec))
     x0 = (np.linalg.cholesky(cov) @ np.random.default_rng(3).normal(size=(n, C))).T
@@ -444,15 +462,16 @@ def test_tensor_core_extended_density(handle, oracle, monkeypatch, n, order, sam
     assert np.array_equal(out['tree_depth'], gen['tree_depth']) and np.array_equal(out['diverging'], gen['diverging'])
 
 
-@pytest.mark.parametrize('family', ['team', 'dmma', 'pair'])
-@pytest.mark.parametrize('env', [{}, {'BFB200_STACK_LEVELS_SMEM': '2'}])
-def test_tensor_core_nuts_deep_trees(handle, oracle, monkeypatch, env, family):
+@pytest.mark.parametrize('family,n', [('dmma', 26), ('pair', 26), ('team', 40)], ids=['dmma', 'pair', 'team-n40'])
+@pytest.mark.parametrize('env', [{}, {'BFB200_STACK_LEVELS_SMEM': '2'}, {'BFB200_STACK_LEVELS_SMEM': '0'}])
+def test_tensor_core_nuts_deep_trees(handle, oracle, monkeypatch, env, family, n):
     """tiny fixed step size: trees reach depth 8-10 (up to 1023 leaves), i.e. every stack level, the L2-resident deep
-    levels, the proposal-slot pool and the depth cap are exercised; outcomes identical to the oracle"""
+    levels, the proposal-slot pool and the depth cap are exercised; outcomes identical to the oracle.  Stack levels in shared
+    memory: the default (team at n = 40: 3), 2, or none but the current subtree (the pair kernel keeps at least one)"""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     monkeypatch.setenv('BFB200_SAMPLER', family)
-    n, C, n_iter = 26, 19, 5
+    C, n_iter = 19, 5
     spec, cov = synthetic_spec(n, 'cubic-2', seed=5)
     handle.set_model(to_device_spec(spec))
     x0 = (np.linalg.cholesky(cov) @ np.random.default_rng(11).normal(size=(n, C))).T
@@ -537,6 +556,24 @@ def test_tensor_core_cubic3_samplers(handle, oracle, monkeypatch, n, sampler, C)
     gen = handle.sampler_run(sampler, n_iter)
     assert handle.sampler_last_path() == 'generic'
     assert np.array_equal(out['tree_depth'], gen['tree_depth']) and np.array_equal(out['diverging'], gen['diverging'])
+
+
+@pytest.mark.parametrize('family,n,order', [('team', 26, 'cubic-2'), ('pair', 10, 'cubic-3')])
+def test_pinned_family_that_cannot_run_the_model_raises(handle, monkeypatch, family, n, order):
+    """BFB200_SAMPLER pins a kernel family; one that has no kernel for the model is an error that names the family, not a
+    silent run on the generic kernel"""
+    from bayesfast_b200._cabi import BfbError
+    spec, cov = synthetic_spec(n, order, seed=3, cubic_scale=0.05)
+    handle.set_model(to_device_spec(spec))
+    C = 16
+    x0 = (np.linalg.cholesky(cov) @ np.random.default_rng(4).normal(size=(n, C))).T
+    handle.sampler_init(cfg_from({}, 4, 8), x0, 0.5, np.ones(n), x0)
+    monkeypatch.setenv('BFB200_SAMPLER', family)
+    with pytest.raises(BfbError, match='BFB200_SAMPLER=%s: the %s kernels cannot run this model' % (family, family)):
+        handle.sampler_run('NUTS', 8)
+    monkeypatch.delenv('BFB200_SAMPLER')
+    handle.sampler_run('NUTS', 8)
+    assert handle.sampler_last_path() == 'dmma'
 
 
 # ---------------------------------------------------------------------------------------------------------------------
