@@ -17,6 +17,17 @@
 #include <cstring>
 #include <map>
 
+// parameters per output: the triangular solve keeps one P-vector in shared memory (128 KB) and a row in registers
+// (32 doubles per thread of 512)
+#define FIT_MAX_P 16384
+
+// opt a kernel in to dynamic shared memory above the default 48 KB (input_size up to 128 needs up to 132 KB)
+template <typename K> static int smem_opt_in(K kernel, size_t bytes)
+{
+    if (bytes > 48 * 1024) BFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    return BFB_OK;
+}
+
 // temporary device allocations of one call: freed on every return path (the error paths used to leak them)
 struct TmpList : std::vector<void *> {
     ~TmpList() { for (void *p : *this) cudaFree(p); }
@@ -90,7 +101,8 @@ __global__ void __launch_bounds__(128) gram_kernel(const double *__restrict__ x,
         for (int b = 0; b < 4; ++b) acc[a][b][0] = acc[a][b][1] = 0.;
     const int64_t r_begin = (int64_t)blockIdx.y * rows_per_chunk;
     const int64_t r_end = min(N, r_begin + rows_per_chunk);
-    // flat, division-free walk over the KC x n block of x (contiguous in global memory): element e = tid + 128 s
+    // flat, division-free walk over the KC x n block of x (contiguous in global memory): element e = tid + 128 s.  The step
+    // (dk, dj) is 128 elements; dj < n, so one wrap per step suffices for every n <= 128 (n > 64: dk = 1, dj = 128 - n)
     const int k_init = tid / n, j_init = tid - k_init * n, dk = 128 / n, dj = 128 - dk * n;
     const int n_el = KC * n;
     for (int64_t r0 = r_begin; r0 < r_end; r0 += KC) {
@@ -167,7 +179,9 @@ __global__ void gram_reduce_kernel(const double *__restrict__ ws, int n_tiles, i
     }
 }
 
-// shifted moments: S1 = sum (x - s), S2 = sum (x - s)(x - s)^T, count.  One block per row range; fixed-order reduce.
+// shifted moments: S1 = sum (x - s), S2 = sum (x - s)(x - s)^T, count.  One block per (row range, slab of MOM_SLAB pairs
+// of S2); the block of slab 0 also sums S1.  Fixed-order reduce.
+#define MOM_SLAB 4096                        // 256 threads x 16 accumulators: one slab for n <= 64, four at n = 128
 __global__ void __launch_bounds__(256) moments_kernel(const double *__restrict__ x, int64_t N, int n,
                                                       const double *__restrict__ shift, int64_t rows_per_block,
                                                       double *__restrict__ ws)
@@ -175,8 +189,8 @@ __global__ void __launch_bounds__(256) moments_kernel(const double *__restrict__
     extern __shared__ double sm[];
     double *xs = sm;   // [64][n+1]
     const int ldx = n + 1, tid = threadIdx.x;
-    const int npair = n * n;
-    const int PER = 16;                      // n <= 64 -> n^2 <= 4096 = 256 * 16
+    const int npair = n * n, pbase = blockIdx.y * MOM_SLAB;
+    const int PER = MOM_SLAB / 256;
     double acc[PER];
 #pragma unroll
     for (int i = 0; i < PER; ++i) acc[i] = 0.;
@@ -192,7 +206,7 @@ __global__ void __launch_bounds__(256) moments_kernel(const double *__restrict__
         __syncthreads();
 #pragma unroll
         for (int i = 0; i < PER; ++i) {
-            int pidx = tid + 256 * i;
+            int pidx = pbase + tid + 256 * i;
             if (pidx < npair) {
                 int a = pidx / n, b = pidx - a * n;
                 double s = acc[i];
@@ -200,7 +214,7 @@ __global__ void __launch_bounds__(256) moments_kernel(const double *__restrict__
                 acc[i] = s;
             }
         }
-        if (tid < n) {
+        if (blockIdx.y == 0 && tid < n) {
             double s = acc1;
             for (int k = 0; k < 64; ++k) s += xs[k * ldx + tid];
             acc1 = s;
@@ -209,10 +223,10 @@ __global__ void __launch_bounds__(256) moments_kernel(const double *__restrict__
     double *out = ws + (size_t)blockIdx.x * (npair + n);
 #pragma unroll
     for (int i = 0; i < PER; ++i) {
-        int pidx = tid + 256 * i;
+        int pidx = pbase + tid + 256 * i;
         if (pidx < npair) out[n + pidx] = acc[i];
     }
-    if (tid < n) out[tid] = acc1;
+    if (blockIdx.y == 0 && tid < n) out[tid] = acc1;
 }
 
 __global__ void moments_reduce_kernel(const double *__restrict__ ws, int n_blocks, int len, double *__restrict__ dst)
@@ -236,7 +250,7 @@ static void push_feat(std::vector<short4> &v, int a, int b, int c, int kind)
 extern "C" int bfb_fit_begin(bfb_handle h, const double *shift)
 {
     BFB_REQUIRE(h && h->has_model, BFB_ERR_STATE, "bfb_fit_begin: set the model (configs) first");
-    BFB_REQUIRE(h->n <= 64, BFB_ERR_ARG, "fit supports input_size <= 64 (got %d)", h->n);
+    BFB_REQUIRE(h->n <= 128, BFB_ERR_ARG, "fit supports input_size <= 128 (got %d)", h->n);
     BFB_CUDA(cudaSetDevice(h->device));
     BFB_CUDA(cudaStreamSynchronize(h->stream));
     bfb_fit_free(h);
@@ -291,7 +305,9 @@ extern "C" int bfb_fit_begin(bfb_handle h, const double *shift)
         g.nt = (g.Pt + TS - 1) / TS;
         g.Ptp = g.nt * TS;
         while ((int)feat.size() < g.Ptp) push_feat(feat, -1, -1, -1, 2);
-        BFB_REQUIRE(g.P <= 16384, BFB_ERR_ARG, "fit: %d parameters per output exceed the single-GPU limit 16384", g.P);
+        BFB_REQUIRE(g.P <= FIT_MAX_P, BFB_ERR_ARG,
+                    "fit: %d parameters per output exceed the limit of %d (full models within it: quadratic up to n = 128, "
+                    "cubic-2 up to n = 104, cubic-3 up to n = 44)", g.P, FIT_MAX_P);
         void *p = nullptr;
         BFB_CUDA(cudaMalloc(&p, sizeof(short4) * feat.size()));
         fs->allocs.push_back(p);
@@ -451,7 +467,8 @@ extern "C" int bfb_fit_accumulate(bfb_handle h, const double *x, const double *y
         n_chunks = (int)((N + rows_per_chunk - 1) / rows_per_chunk);
         int rc = ensure_ws(fs, (size_t)n_tiles * n_chunks * TS * TS);
         if (rc) return rc;
-        size_t smem = sizeof(double) * (KC * (n + 2) + KC + 2 * KC * LDP);
+        size_t smem = sizeof(double) * (KC * (n + 2) + KC + 2 * KC * LDP);     // 68 KB at n = 128
+        if ((rc = smem_opt_in(gram_kernel, smem))) return rc;
         dim3 grid(n_tiles, n_chunks);
         gram_kernel<<<grid, 128, smem, h->stream>>>(dx, dy, dw, N, n, m, g.d_feat, g.nt, rows_per_chunk, fs->ws);
         h->launches++;
@@ -468,7 +485,9 @@ extern "C" int bfb_fit_accumulate(bfb_handle h, const double *x, const double *y
         const int len = n * n + n;
         int rc = ensure_ws(fs, (size_t)nb * len);
         if (rc) return rc;
-        moments_kernel<<<nb, 256, sizeof(double) * 64 * (n + 1), h->stream>>>(dx, N, n, fs->d_shift, rpb, fs->ws);
+        const size_t smem = sizeof(double) * 64 * (n + 1);                     // 65 KB at n = 128
+        if ((rc = smem_opt_in(moments_kernel, smem))) return rc;
+        moments_kernel<<<dim3(nb, (n * n + MOM_SLAB - 1) / MOM_SLAB), 256, smem, h->stream>>>(dx, N, n, fs->d_shift, rpb, fs->ws);
         h->launches++;
         BFB_CUDA(cudaGetLastError());
         moments_reduce_kernel<<<(len + 255) / 256, 256, 0, h->stream>>>(fs->ws, nb, len, fs->buf + fs->off_s1);
@@ -558,9 +577,10 @@ extern "C" int bfb_fit_max_beta(bfb_handle h, const double *x, int64_t N, const 
         if (beta_out && (rc = dmal(sizeof(double) * N, &dbeta))) return rc;
     }
     int blocks = (int)std::min<int64_t>((N + 3) / 4, (int64_t)h->sm_count * 16);
-    beta_kernel<<<blocks, 128, sizeof(double) * (n * n + 4 * n), h->stream>>>((const double *)dxv, N, n, (const double *)dmu,
-                                                                              (const double *)dh, (double *)dbeta,
-                                                                              (unsigned long long *)dmax);
+    const size_t smem = sizeof(double) * (n * n + 4 * n);                     // 132 KB at n = 128
+    if ((rc = smem_opt_in(beta_kernel, smem))) return rc;
+    beta_kernel<<<blocks, 128, smem, h->stream>>>((const double *)dxv, N, n, (const double *)dmu, (const double *)dh,
+                                                  (double *)dbeta, (unsigned long long *)dmax);
     h->launches++;
     BFB_CUDA(cudaGetLastError());
     unsigned long long bits = 0;
@@ -696,78 +716,86 @@ __global__ void transpose_lower_kernel(const double *__restrict__ L, int P, doub
     if (ii < P && jj < P) U[(size_t)ii * P + jj] = t[threadIdx.x][threadIdx.y];
 }
 
-// one CTA per right-hand side: L z = b (using U = L^T for coalesced rows), then L^T c = z.  Column-oriented substitution: step j
-// fixes one unknown and updates the rest with one AXPY over a row of U (of L on the way back), one barrier per step.  The row of
-// step j + 1 is loaded into registers while step j runs (the steps are latency bound: 2 P dependent steps, each a barrier, a shared-
-// memory read, a division and the row load -- unpipelined the L2 latency of that load was most of the 1.7 ms at P = 1054).
-__global__ void __launch_bounds__(1024) chol_solve_kernel(const double *__restrict__ L, const double *__restrict__ U, int P,
-                                                          const double *__restrict__ B, int nr, double *__restrict__ X)
+// one CTA per right-hand side: L z = b (using U = L^T for coalesced rows), then L^T c = z, both in place in ONE P-vector of
+// shared memory (128 KB at P = 16384).  Column-oriented substitution: step j fixes one unknown and updates the rest with one AXPY
+// over a row of U (of L on the way back), one barrier per step.  Thread 0 stores the unknown of step j into z[j] after the barrier
+// of step j + 1, when no thread reads that slot any more.  Each row element of step j + 1 is loaded into the register that the
+// update of step j has just consumed, so the loads are in flight across the next barrier with PF registers, not 2 PF (the
+// steps are latency bound: 2 P dependent steps, each a barrier, a shared-memory read, a division and the row load -- unpipelined
+// the L2 latency of that load was most of the 1.7 ms at P = 1054).  PF row elements per thread: P <= PF * 1024.  Which
+// thread updates an element does not change its sequence of fused multiply-adds, so every PF gives the same result.
+template <int NT, int PF>
+__global__ void __launch_bounds__(NT) chol_solve_kernel(const double *__restrict__ L, const double *__restrict__ U, int P,
+                                                        const double *__restrict__ B, int nr, double *__restrict__ X)
 {
-    extern __shared__ double sm[];
-    double *z = sm, *o = sm + P;
-    const int col = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
-    constexpr int PF = 4;                                   // row elements per thread held in registers: P <= PF * blockDim.x
+    extern __shared__ double z[];
+    constexpr int nt = NT;                                  // blockDim.x: constant row offsets of the register-held elements
+    const int col = blockIdx.x, tid = threadIdx.x;
     for (int i = tid; i < P; i += nt) z[i] = B[(size_t)i * nr + col];
-    if (P > PF * nt) {                                      // (not reached: the fit caps P far below) unpipelined fall-back
-        for (int j = 0; j < P; ++j) {
-            __syncthreads();
-            const double zj = z[j] / U[(size_t)j * P + j];
-            if (tid == 0) o[j] = zj;
-            const double *Uj = U + (size_t)j * P;
-            for (int i = j + 1 + tid; i < P; i += nt) z[i] = fma(-Uj[i], zj, z[i]);
-        }
+    double u[PF], d = U[0], prev = 0.;                     // row 0 of U right of the diagonal, and the diagonal
+#pragma unroll
+    for (int e = 0; e < PF; ++e) { const int i = 1 + tid + e * nt; u[e] = (i < P) ? U[i] : 0.; }
+    for (int j = 0; j < P; ++j) {
         __syncthreads();
-        for (int j = P - 1; j >= 0; --j) {
-            __syncthreads();
-            const double cj = o[j] / L[(size_t)j * P + j];
-            if (tid == 0) z[j] = cj;
-            const double *Lj = L + (size_t)j * P;
-            for (int k = tid; k < j; k += nt) o[k] = fma(-Lj[k], cj, o[k]);
-        }
-    } else {
-        double u[PF], d;
-        auto load_u = [&](int j) {                          // row j of U right of the diagonal, and the diagonal
-            const double *Uj = U + (size_t)j * P;
-            d = Uj[j];
+        const double zj = z[j] / d;
+        if (tid == 0 && j > 0) z[j - 1] = prev;
+        prev = zj;
+        const double *Un = U + (size_t)min(j + 1, P - 1) * P;
+        d = Un[min(j + 1, P - 1)];
 #pragma unroll
-            for (int e = 0; e < PF; ++e) { const int i = j + 1 + tid + e * nt; u[e] = (i < P) ? Uj[i] : 0.; }
-        };
-        load_u(0);
-        for (int j = 0; j < P; ++j) {
-            __syncthreads();
-            const double zj = z[j] / d;
-            if (tid == 0) o[j] = zj;
-            double un[PF];
-#pragma unroll
-            for (int e = 0; e < PF; ++e) un[e] = u[e];
-            const int jn = (j + 1 < P) ? j + 1 : j;
-            load_u(jn);                                     // in flight across the barrier of the next step
-#pragma unroll
-            for (int e = 0; e < PF; ++e) { const int i = j + 1 + tid + e * nt; if (i < P) z[i] = fma(-un[e], zj, z[i]); }
-        }
-        __syncthreads();
-        auto load_l = [&](int j) {                          // row j of L left of the diagonal, and the diagonal
-            const double *Lj = L + (size_t)j * P;
-            d = Lj[j];
-#pragma unroll
-            for (int e = 0; e < PF; ++e) { const int k = tid + e * nt; u[e] = (k < j) ? Lj[k] : 0.; }
-        };
-        load_l(P - 1);
-        for (int j = P - 1; j >= 0; --j) {
-            __syncthreads();
-            const double cj = o[j] / d;
-            if (tid == 0) z[j] = cj;                        // z now collects the solution
-            double un[PF];
-#pragma unroll
-            for (int e = 0; e < PF; ++e) un[e] = u[e];
-            const int jn = (j > 0) ? j - 1 : 0;
-            load_l(jn);
-#pragma unroll
-            for (int e = 0; e < PF; ++e) { const int k = tid + e * nt; if (k < j) o[k] = fma(-un[e], cj, o[k]); }
+        for (int e = 0; e < PF; ++e) {
+            const int i = j + 1 + tid + e * nt;
+            if (i < P) z[i] = fma(-u[e], zj, z[i]);
+            u[e] = (i + 1 < P) ? Un[i + 1] : 0.;            // row j + 1: in flight across the barrier of the next step
         }
     }
+    if (tid == 0) z[P - 1] = prev;
+    __syncthreads();
+    const double *Ll = L + (size_t)(P - 1) * P;             // row P - 1 of L left of the diagonal, and the diagonal
+    d = Ll[P - 1];
+#pragma unroll
+    for (int e = 0; e < PF; ++e) { const int k = tid + e * nt; u[e] = (k < P - 1) ? Ll[k] : 0.; }
+    for (int j = P - 1; j >= 0; --j) {
+        __syncthreads();
+        const double cj = z[j] / d;
+        if (tid == 0 && j < P - 1) z[j + 1] = prev;
+        prev = cj;
+        const double *Ln = L + (size_t)max(j - 1, 0) * P;
+        d = Ln[max(j - 1, 0)];
+#pragma unroll
+        for (int e = 0; e < PF; ++e) {
+            const int k = tid + e * nt;
+            if (k < j) z[k] = fma(-u[e], cj, z[k]);
+            u[e] = (k < j - 1) ? Ln[k] : 0.;
+        }
+    }
+    if (tid == 0) z[0] = prev;
     __syncthreads();
     for (int i = tid; i < P; i += nt) X[(size_t)i * nr + col] = z[i];
+}
+
+template <int NT, int PF>
+static int chol_solve_launch(bfb_context *h, const double *L, const double *U, int P, const double *B, int nr, double *X)
+{
+    const size_t smem = sizeof(double) * P;
+    int rc;
+    if ((rc = smem_opt_in(chol_solve_kernel<NT, PF>, smem))) return rc;
+    chol_solve_kernel<NT, PF><<<nr, NT, smem, h->stream>>>(L, U, P, B, nr, X);
+    return BFB_OK;
+}
+
+// the triangular solves of every right-hand side (B, X: P x nr).  Above P = 8192 a row takes 16 registers per thread of 1024,
+// more than the 64 registers a thread of 1024 has without spilling; 512 threads hold it in 32.
+static int chol_solve(bfb_context *h, const double *L, const double *U, int P, const double *B, int nr, double *X)
+{
+    static_assert(FIT_MAX_P <= 512 * 32, "chol_solve_kernel<512, 32> holds a row of at most 16384");
+    const int rc = P <= 4096 ? chol_solve_launch<1024, 4>(h, L, U, P, B, nr, X)
+                 : P <= 8192 ? chol_solve_launch<1024, 8>(h, L, U, P, B, nr, X)
+                             : chol_solve_launch<512, 32>(h, L, U, P, B, nr, X);
+    if (rc) return rc;
+    h->launches++;
+    BFB_CUDA(cudaGetLastError());
+    return BFB_OK;
 }
 
 // R = Bs - As * X   (As symmetric P x P, X and Bs are P x nr); one warp per (row, rhs)
@@ -834,16 +862,13 @@ extern "C" int bfb_fit_solve(bfb_handle h, double *coef_out, double *rel_resid)
         if ((rc = cholesky_device(h, A, P, d_info))) return rc;
         transpose_lower_kernel<<<dim3((P + 31) / 32, (P + 31) / 32), dim3(32, 32), 0, h->stream>>>(A, P, U);
         h->launches++;
-        const size_t smem = sizeof(double) * 2 * P;
-        BFB_CUDA(cudaFuncSetAttribute(chol_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        chol_solve_kernel<<<nr, 1024, smem, h->stream>>>(A, U, P, Bs, nr, X);
-        h->launches++;
+        if ((rc = chol_solve(h, A, U, P, Bs, nr, X))) return rc;
         const int64_t nw = (int64_t)P * nr;
         for (int it = 0; it < 2; ++it) {      // iterative refinement on the equilibrated system
             residual_kernel<<<(unsigned)((nw + 3) / 4), 128, 0, h->stream>>>(As, P, X, Bs, nr, R);
-            chol_solve_kernel<<<nr, 1024, smem, h->stream>>>(A, U, P, R, nr, D);
+            if ((rc = chol_solve(h, A, U, P, R, nr, D))) return rc;
             axpy_kernel<<<(unsigned)((nw + 255) / 256), 256, 0, h->stream>>>(X, D, nw);
-            h->launches += 3;
+            h->launches += 2;
         }
         residual_kernel<<<(unsigned)((nw + 3) / 4), 128, 0, h->stream>>>(As, P, X, Bs, nr, R);
         h->launches++;

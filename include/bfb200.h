@@ -112,6 +112,10 @@ int bfb_set_prior(bfb_handle h, const double *w, const double *mu, double c0);
  * Rows may be accumulated in several calls (and on several GPUs: bfb_fit_export/import carry the
  * packed partial sums through an all-reduce).  The model set by bfb_set_model supplies the configs
  * (coefficients there are ignored).  y [N,m]; w NULL or [N] (rows are scaled by w like poly.py:566-568).
+ * Limits, checked by bfb_fit_begin (BFB_ERR_ARG): input_size <= 128, the evaluators' limit, and P <= 16384 parameters per
+ * output (the configs serving one output together): full quadratic models up to n = 128 (P = 8385), cubic-2 up to n = 104
+ * (P = 16381), cubic-3 up to n = 44 (P = 16215).  The bound and decay ellipsoids (bfb_fit_moments, bfb_fit_max_beta) take
+ * input_size <= 128.
  * ---------------------------------------------------------------------------------------------- */
 int bfb_fit_begin(bfb_handle h, const double *shift /* [n] or NULL: reference point of the shifted moments, identical on all ranks */);
 int bfb_fit_accumulate(bfb_handle h, const double *x, const double *y, const double *w, int64_t N, int loc);
